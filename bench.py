@@ -2,6 +2,7 @@
 """bench.py -- headline benchmark of the purification hot path (BASELINE.json).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload purify|pgd|gender|cars] [--extras 0|1]
+                  [--dump-outputs DIR]
 
 "step" = one pass of the hot path over one batch of synthetic input:
   workload purify (default, BASELINE configs[1]): NVAE CelebA-64 "ids" + configs/ours_learned_blur_ids.yaml
@@ -25,6 +26,9 @@ The JSON line (one, on stdout, rank 0):
             (configs[4], short run, at every N), and at N = 1 `gender`, `cars` (configs[2], [3]) and `incumbent_gpu` (the UNMODIFIED
             reference modules on cuda:0 -- fp32 as the reference runs them, and under bf16 autocast -- the bar the kernels must beat).
 --impl reference: the reference's own CPU implementation of the path on the host cores, same config, bounded sample per step.
+--dump-outputs DIR: after the timed steps, what the last timed step returned to its caller (logits; for pgd the success flags, L-inf
+            distances and adversarial images) as DIR/<name>.npy in float32, at most 64 MB in all.  Inputs, weights and the noise seeds
+            are seeded, so two builds run with the same arguments can be compared output for output.
 Multi-GPU (torchrun): batch sharded data-parallel, no data-path collective; the only collective is one
 all-reduce of the int64[3] accuracy counters (SURVEY 8e).  scaling = weak (fixed 512 images per GPU).
 """
@@ -234,7 +238,7 @@ def incumbent_gpu(dev, workloads=("purify", "gender", "cars"), ours=None):
     from gen_adversarial_b200 import synth
     out = {}
     if not ref_import.reference_available():
-        return {"unavailable": "reference tree absent (run oracle/build_ref.sh in the build container)"}
+        return {"unavailable": "reference tree absent (set GA_REFERENCE_ROOT or run oracle/build_ref.sh)"}
     torch.backends.cudnn.benchmark = True
     for wl in workloads:
         try:
@@ -324,8 +328,10 @@ class Ctx:
         return float(t.item())
 
 
-def measure(ctx, dm, workload, B, steps, warmup, mode, use_graph, pgd_steps=50, sample_clocks=False, global_offset=None):
-    """resident + end-to-end timing of one workload -> dict (identical on every rank)"""
+def measure(ctx, dm, workload, B, steps, warmup, mode, use_graph, pgd_steps=50, sample_clocks=False, global_offset=None,
+            keep_outputs=False):
+    """resident + end-to-end timing of one workload -> dict (identical on every rank); keep_outputs: "_outputs" holds host copies of
+    what the last resident timed step returned"""
     from gen_adversarial_b200 import ops, synth, graphs as ga_graphs
     dev, rank, world = ctx.dev, ctx.rank, ctx.world
     pgd = workload == "pgd"
@@ -347,13 +353,13 @@ def measure(ctx, dm, workload, B, steps, warmup, mode, use_graph, pgd_steps=50, 
 
     def step_resident():
         if pgd:
-            succ, _, _ = attack(x_dev, y_dev, dm)
+            succ, linf, adv = attack(x_dev, y_dev, dm)
             counters[2] += (~succ).sum()
-            return succ
+            return {"success": succ, "linf": linf, "x_adv": adv}
         with torch.no_grad():
             logits = dm(x_dev)
         ops.softmax_xent(logits, y_dev, want_grad=False, counter=counters[1:2].view(torch.int64))
-        return logits
+        return {"logits": logits}
 
     def step_e2e():
         xd = x_host.to(dev, non_blocking=True)
@@ -383,10 +389,12 @@ def measure(ctx, dm, workload, B, steps, warmup, mode, use_graph, pgd_steps=50, 
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(steps):
-        step_resident()
+        out = step_resident()
     e1.record()
     ctx.barrier()
     ms = ctx.max_over_ranks(e0.elapsed_time(e1))
+    # copied before the next call: a replayed CUDA graph returns static buffers that the next call overwrites
+    outputs = {k: v.detach().to(torch.float32).cpu() for k, v in out.items()} if keep_outputs else None
     clocks = sampler.stop() if sampler else None
     launches = ops.launch_count(reset=True) + ga_graphs.REPLAYED_LAUNCHES[0] - replayed0      # eager launches + graph-replayed kernel nodes
     counters[0] = B * steps
@@ -413,7 +421,29 @@ def measure(ctx, dm, workload, B, steps, warmup, mode, use_graph, pgd_steps=50, 
             "cuda_graph": bool(use_graph), "gflop_per_image_algorithmic": gflop, "tflops_algorithmic": value * gflop / 1e3,
             "counters": {"n_total": int(counters[0].item()), "n_clean_correct": int(counters[1].item()),
                          "n_robust_correct": int(counters[2].item())},
-            "_x_dev": x_dev, "_y_dev": y_dev}
+            "_x_dev": x_dev, "_y_dev": y_dev, "_outputs": outputs}
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, outputs, rank, world):
+    """outputs {name: host tensor, batch first} -> path/<name>.npy in float32 (name_rank<r>.npy on a multi-GPU run).  Above
+    DUMP_LIMIT_BYTES in all (over the ranks), every array keeps the same seeded sample of batch rows, listed in sample_rows.npy."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    budget = DUMP_LIMIT_BYTES // world - 4096                        # room for the .npy headers
+    n = next(iter(outputs.values())).shape[0]
+    row_bytes = sum(v[0].numel() * 4 for v in outputs.values())
+    if n * row_bytes > budget:
+        keep = budget // (row_bytes + 8)                             # + 8: the float64 row index
+        rows = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:keep].sort().values
+        outputs = {k: v[rows] for k, v in outputs.items()}
+        outputs["sample_rows"] = rows.to(torch.float64)
+    suffix = f"_rank{rank}" if world > 1 else ""
+    for k, v in outputs.items():
+        np.save(os.path.join(path, f"{k}{suffix}.npy"), v.numpy())
+    log(f"[bench] outputs of the last timed step -> {path}: " + ", ".join(f"{k}{tuple(v.shape)}" for k, v in outputs.items()))
 
 
 def instrumented_pass(ctx, dm, workload, x_dev, y_dev, steps, step_ms, breakdown=False):
@@ -522,11 +552,17 @@ def run_ours(args):
     B = args.batch if args.batch is not None else DEFAULT_BATCH[wl]
     use_graph = (args.cuda_graph == 1) or (args.cuda_graph < 0 and (pgd or wl == "purify"))
     t_start = time.perf_counter()
+    # every call draws its Philox noise seed from torch's CPU generator, which torch seeds at random in each process: a fixed seed
+    # makes two runs with the same arguments compute the same outputs
+    torch.manual_seed(0)
     dm = make_ours(wl, mode, dev, args.chunk)
     n_streams = args.streams if args.streams > 0 else (2 if wl in ("purify", "pgd") else 1)
     dm.set_streams(n_streams)              # public API: no-grad calls run as part-batches on CUDA streams (results unchanged)
-    main = measure(ctx, dm, wl, B, args.steps, args.warmup, mode, use_graph and not sg, args.pgd_steps, sample_clocks=True)
+    main = measure(ctx, dm, wl, B, args.steps, args.warmup, mode, use_graph and not sg, args.pgd_steps, sample_clocks=True,
+                   keep_outputs=bool(args.dump_outputs))
     log(f"[bench] {wl}: {main['value']:.1f} img/s resident, {main['e2e']['value']:.1f} e2e ({time.perf_counter() - t_start:.0f} s)")
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, main.pop("_outputs"), rank, world)
     roof, extra = None, []
     if not sg or args.breakdown:
         dm.set_streams(1)                  # per-launch events: one stream, so a launch's duration is its own
@@ -635,8 +671,14 @@ def main():
     ap.add_argument("--ref-batch", type=int, default=0, help="bounded sample per step of the CPU reference arm (default 64 ids / 2 StyleGAN)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--breakdown", action="store_true", help="CUDA-event time of EVERY op of the instrumented pass (table on stderr)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float32, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs needs --impl ours: the reference arm draws fresh noise on every call")
         args.steps = args.steps if args.steps is not None else 4
         args.warmup = args.warmup if args.warmup is not None else 1
         run_reference(args)

@@ -1,6 +1,9 @@
 """TEST INFRASTRUCTURE ONLY -- generates tests/golden/*.pt by running the UNMODIFIED reference
-(imported from /root/reference through oracle/ref_import.py) on seeded synthetic checkpoints,
-inputs and explicit noise.  Run in the build container:  python -m oracle.make_golden
+(located by oracle/ref_import.py) on seeded synthetic checkpoints, inputs and explicit noise.
+Run where the reference is available:  python -m oracle.make_golden
+
+No fixture may exceed 1 MB: seeded weights are stored as their seed, layout and digest (load_nvae_tiny),
+and a large `purified` tensor as a fixed, seeded sample of its elements (stored_purified).
 
 The reference ships no golden vectors (SURVEY.md section 4), so these fixtures -- outputs of the
 reference's own `NVAEDefenseModel.__call__` (src/defenses/ours/abstract_models.py:161-193,
@@ -16,6 +19,7 @@ import shutil
 import sys
 import tempfile
 
+import numpy as np
 import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -44,6 +48,41 @@ def sd_digest(sd) -> str:
         h.update(k.encode())
         h.update(sd[k].detach().cpu().contiguous().numpy().tobytes())
     return h.hexdigest()
+
+
+PURIFIED_KEEP = 196608          # elements of a sampled `purified` (half of the 2 x 3 x 256 x 256 E4E output: 786 KB in float32)
+
+
+def _sample_index(numel: int, keep: int, seed: int) -> torch.Tensor:
+    # numpy's legacy RandomState stream is frozen across releases, so the positions never move
+    return torch.from_numpy(np.sort(np.random.RandomState(seed).permutation(numel)[:keep]).astype(np.int64))
+
+
+def sample_purified(out: dict, keep: int = PURIFIED_KEEP, seed: int = 0) -> dict:
+    """replace out["purified"] by a seeded sample of `keep` of its elements (full float32 precision)"""
+    pur = out.pop("purified")
+    idx = _sample_index(pur.numel(), keep, seed)
+    out.update(purified_shape=tuple(pur.shape), purified_seed=seed, purified_sample=pur.flatten()[idx].clone())
+    return out
+
+
+def stored_purified(g: dict, pur: torch.Tensor):
+    """-> (pur at the positions the fixture stores, the reference's values there): all of `purified`, or its seeded sample"""
+    if "purified" in g:
+        return pur, g["purified"]
+    assert tuple(pur.shape) == tuple(g["purified_shape"]), (tuple(pur.shape), g["purified_shape"])
+    idx = _sample_index(pur.numel(), g["purified_sample"].numel(), g["purified_seed"])
+    return pur.reshape(-1)[idx.to(pur.device)], g["purified_sample"]
+
+
+def load_nvae_tiny(path: str) -> dict:
+    """tests/golden/nvae_tiny.pt with its "state_dict" regenerated from the stored seed and checked against the stored digest"""
+    from gen_adversarial_b200 import synth
+    g = torch.load(path, weights_only=True)
+    sd = synth.make_nvae_state_dict(g["cfg"], g["resolution"], seed=g["state_dict_seed"])
+    assert sd_digest(sd) == g["state_dict_digest"], "synth.make_nvae_state_dict no longer gives the weights the fixture was made with"
+    g["state_dict"] = sd
+    return g
 
 
 class _MeanClassifier:
@@ -98,7 +137,7 @@ def run_reference_stylegan(kind: str, batch: int = 2):
 
 def main_stylegan_paths():
     os.makedirs(GOLDEN, exist_ok=True)
-    torch.save(run_reference_stylegan("e4e"), os.path.join(GOLDEN, "e4e_gender_b2.pt"))
+    torch.save(sample_purified(run_reference_stylegan("e4e")), os.path.join(GOLDEN, "e4e_gender_b2.pt"))
     torch.save(run_reference_stylegan("trans"), os.path.join(GOLDEN, "trans_cars_b2.pt"))
     shutil.rmtree(SCRATCH, ignore_errors=True)
 
@@ -169,7 +208,9 @@ def main():
         _, pur = run_reference_nvae(ckpt, alphas, att, eps, blur, x, noises)
         cases.append({"name": name, "alphas": alphas, "attenuation": att, "eps": eps, "blur": blur, "purified": pur})
         print("tiny", name, pur.mean().item(), pur.std().item())
-    torch.save({"cfg": cfg, "resolution": res, "state_dict": ckpt["state_dict_temp=0.6"], "x": x,
+    sd = ckpt["state_dict_temp=0.6"]
+    torch.save({"cfg": cfg, "resolution": res, "state_dict_seed": 3, "state_dict_digest": sd_digest(sd),
+                "state_dict_layout": {k: tuple(v.shape) for k, v in sd.items()}, "x": x,
                 "noises": noises, "cases": cases}, os.path.join(GOLDEN, "nvae_tiny.pt"))
 
     # ---------------------------------------------------------------- C32 + VGG11 (weights regenerated from seeds)

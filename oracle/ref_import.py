@@ -33,6 +33,7 @@ import importlib
 import math
 import os
 import sys
+import tempfile
 import types
 import typing
 
@@ -207,9 +208,15 @@ def install(cpu_stylegan_ops: bool = True):
         return
     if not reference_available():
         raise RuntimeError(f"reference tree not found at {REFERENCE_ROOT} (only present in the build container)")
-    # keep any torch JIT cache inside the repo (oracle/_ref is git-ignored)
-    os.environ.setdefault("TORCH_EXTENSIONS_DIR",
-                          os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref", "torch_ext"))
+    # keep any torch JIT cache inside the repo (oracle/_ref is git-ignored); a read-only tree gets a per-run temporary directory
+    if "TORCH_EXTENSIONS_DIR" not in os.environ:
+        ext = os.path.join(_HERE, "_ref", "torch_ext")
+        try:
+            os.makedirs(ext, exist_ok=True)
+            writable = os.access(ext, os.W_OK)
+        except OSError:
+            writable = False
+        os.environ["TORCH_EXTENSIONS_DIR"] = ext if writable else tempfile.mkdtemp(prefix="ga_torch_ext_")
     builtins.Union = typing.Union                                             # shim 1
     _install_kornia()                                                         # shim 3
     if REFERENCE_ROOT not in sys.path:

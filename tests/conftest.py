@@ -26,8 +26,8 @@ GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 @pytest.fixture(scope="session")
 def golden_tiny():
-    import torch
-    return torch.load(os.path.join(GOLDEN, "nvae_tiny.pt"), weights_only=True)
+    from oracle.make_golden import load_nvae_tiny
+    return load_nvae_tiny(os.path.join(GOLDEN, "nvae_tiny.pt"))
 
 
 @pytest.fixture(scope="session")
