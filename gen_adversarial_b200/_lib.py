@@ -168,6 +168,12 @@ _PROTOS = {
     "ga_upfirdn2d": (c_int, [T, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, T, c_void_p]),
     "ga_avgpool_to_nchw": (c_int, [T, c_int, c_int, c_void_p, c_void_p]),
     "ga_latent_lerp": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "ga_styled_bias_act_bwd_parts": (c_int, [c_int, c_int]),
+    "ga_styled_bias_act_bwd": (c_int, [T, T, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_void_p, c_int, T,
+                                       c_void_p, c_void_p, c_void_p, c_void_p]),
+    "ga_style_bwd": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "ga_latent_lerp_bwd": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
+    "ga_image_pool_out_bwd": (c_int, [c_void_p, T, c_int, c_int, c_int, c_float, T, c_void_p]),
     "ga_apgd_l2_step": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_float, c_float, c_int, c_int, c_void_p]),
     "ga_fgsm_l2_step": (c_int, [c_void_p, c_void_p, c_float, c_void_p, c_int, c_int, c_void_p]),
     "ga_l2_ball_start": (c_int, [c_void_p, c_void_p, c_float, c_void_p, c_int, c_int, c_void_p]),

@@ -55,6 +55,42 @@ class Tape:
         (self.vgg if rec[0].startswith(("vgg_", "resnet")) else self.nvae).append(rec)
 
 
+class CodesTape:
+    """what `_StyleGanDefenseBase._from_codes_cuda` leaves behind: the generator's tape, the classifier's records, the mixing alphas"""
+
+    def __init__(self):
+        from .stylegan_engine import SynthesisTape
+        self.syn = SynthesisTape()
+        self.cls = []
+        self.alphas = None
+
+
+class _CodesFn(torch.autograd.Function):
+    """`from_codes` of a StyleGAN defense as ONE node: W+ codes -> mix -> generator -> pool -> classifier.  Same contract as _DefenseFn:
+    the forward tapes, the backward runs the dgrad-only reverse sweep and leaves the tape intact (repeated backward works)."""
+
+    @staticmethod
+    def forward(ctx, codes, model):
+        tape = CodesTape()
+        with torch.no_grad():
+            preds, purified = model._from_codes_cuda(codes.detach(), tape=tape)
+        ctx.tape, ctx.model = tape, model
+        ctx.set_materialize_grads(False)
+        return preds, purified
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, g_preds, g_purified):
+        if g_preds is None and g_purified is None:
+            return None, None
+        return ctx.model._from_codes_backward(ctx.tape, g_preds, g_purified), None
+
+
+def codes_apply(model, codes: torch.Tensor):
+    """differentiable `_StyleGanDefenseBase.from_codes` body -> (preds, purified)"""
+    return _CodesFn.apply(codes, model)
+
+
 def defense_apply(model, batch: torch.Tensor):
     """differentiable `MLVGMDefenseModel.__call__` body -> (preds, purified)"""
     return _DefenseFn.apply(batch, model)

@@ -353,6 +353,173 @@ __global__ void latent_lerp_kernel(const float* __restrict__ codes, const float*
   out[i] = (1.f - a) * codes[i] + a * styles[i];
 }
 
+// ============================================================================ input-gradient backward of the generator (W+ decode half)
+// Partial per-(sample, channel) sums over FIXED pixel slices: a slice holds ~32K elements whatever the batch, so every reduction runs
+// in the same order for a sample wherever it sits in the batch (bit-reproducible, no atomics; DESIGN §3).
+static int sba_bwd_pix_per_part(int c) { return c >= 32768 ? 1 : 32768 / c; }
+
+struct SbaBwd {
+  const void* v; int v_dtype;                          // taped activation act(pre) [n][h][w][c]
+  const void* g_next; int g_next_dtype;                // gradient w.r.t. the next conv's (modulated) input [n][h][w][c], nullable
+  const float* s_next;                                 // [n][c] the next conv's style, nullable
+  const float* g_rgb; const float* w_rgb;              // ToRGB output gradient [n][h][w][4] fp32 and its weights [c][4] fp32, nullable
+  const float* s_rgb;                                  // [n][c]
+  const float* demod; const float* noise; float noise_w; const float* bias;
+  void* g_y; int g_y_dtype; int phases;                // conv-output gradient, nullable (dots only)
+  float* dot_next; float* dot_rgb; float* dot_demod;   // [n][parts][c], nullable
+  int H, W, C, ppp, parts;
+};
+
+// Mirror of styled_bias_act (+ the 1x1 ToRGB adjoint of torgb_fused) for one styled layer, one pass:
+//   g_v   = s_next * g_next + s_rgb * (W_rgb^T g_rgb)
+//   g_pre = g_v * lrelu'(pre) * sqrt(2)                 (sign of the taped activation = sign of pre)
+//   g_y   = g_pre * demod                               (phase-major [n][h/2][w/2][4c] for up-sampling layers)
+//   dots:  sum g_next * v (d s_next),  sum (W_rgb^T g_rgb) * v (d s_rgb),  sum g_pre * u = demod * d demod,  u = pre - bias - noise,
+//          pre recovered by inverting the leaky ReLU of v (no division by demod or s).
+// grid (parts, n); thread = (4-channel group, pixel lane); lanes reduce through shared memory in a fixed order.
+__global__ void __launch_bounds__(256) styled_bias_act_bwd_kernel(const SbaBwd p) {
+  extern __shared__ float sm[];                        // [C][4] ToRGB weights, then 3 x [256][4] partial sums
+  float4* s_w = reinterpret_cast<float4*>(sm);
+  float* red = sm + (p.w_rgb != nullptr ? p.C * 4 : 0);
+  if (p.w_rgb != nullptr)
+    for (int c = threadIdx.x; c < p.C; c += 256) s_w[c] = __ldg(reinterpret_cast<const float4*>(p.w_rgb) + c);
+  __syncthreads();
+  const int c4n = p.C >> 2, lanes = 256 / c4n;
+  const int cg = threadIdx.x % c4n, lane = threadIdx.x / c4n, c = cg * 4;
+  const int part = blockIdx.x;
+  const int64_t n = blockIdx.y;
+  const int HW = p.H * p.W;
+  const int p0 = part * p.ppp, p1 = min(HW, p0 + p.ppp);
+  const float kpos = 1.4142135623730951f, kneg = 0.2f * 1.4142135623730951f;
+  float sn[4] = {0.f, 0.f, 0.f, 0.f}, sr[4] = {0.f, 0.f, 0.f, 0.f}, dm[4] = {1.f, 1.f, 1.f, 1.f}, bs[4] = {0.f, 0.f, 0.f, 0.f};
+  for (int j = 0; j < 4; ++j) {
+    if (p.s_next) sn[j] = p.s_next[n * p.C + c + j];
+    if (p.g_rgb) sr[j] = p.s_rgb[n * p.C + c + j];
+    if (p.demod) dm[j] = p.demod[n * p.C + c + j];
+    if (p.bias) bs[j] = p.bias[c + j];
+  }
+  float a_next[4] = {0.f, 0.f, 0.f, 0.f}, a_rgb[4] = {0.f, 0.f, 0.f, 0.f}, a_dem[4] = {0.f, 0.f, 0.f, 0.f};
+  for (int pix = p0 + lane; pix < p1; pix += lanes) {
+    const int64_t o = (n * HW + pix) * p.C + c;
+    float v[4], gv[4] = {0.f, 0.f, 0.f, 0.f};
+    ld4s(p.v, p.v_dtype, o, v);
+    if (p.g_next) {
+      float gn[4];
+      ld4s(p.g_next, p.g_next_dtype, o, gn);
+#pragma unroll
+      for (int j = 0; j < 4; ++j) { gv[j] = fmaf(sn[j], gn[j], gv[j]); a_next[j] = fmaf(gn[j], v[j], a_next[j]); }
+    }
+    if (p.g_rgb) {
+      const float4 gr = __ldg(reinterpret_cast<const float4*>(p.g_rgb + (n * HW + pix) * 4));
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const float4 w = s_w[c + j];
+        const float t = w.x * gr.x + w.y * gr.y + w.z * gr.z + w.w * gr.w;
+        gv[j] = fmaf(sr[j], t, gv[j]);
+        a_rgb[j] = fmaf(t, v[j], a_rgb[j]);
+      }
+    }
+    if (p.g_y == nullptr) continue;
+    float gy[4];
+    const float nz = p.noise != nullptr ? p.noise_w * __ldg(p.noise + pix) : 0.f;
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      const bool pos = v[j] > 0.f;
+      const float gp = gv[j] * (pos ? kpos : kneg);
+      const float pre = v[j] * (pos ? 1.f / kpos : 1.f / kneg);
+      a_dem[j] = fmaf(gp, pre - nz - bs[j], a_dem[j]);
+      gy[j] = gp * dm[j];
+    }
+    int64_t dst = o;
+    if (p.phases) {
+      const int x = pix % p.W, yy = pix / p.W;
+      const int ph = (yy & 1) * 2 + (x & 1);
+      dst = (((n * (p.H >> 1) + (yy >> 1)) * (p.W >> 1) + (x >> 1)) * 4 + ph) * p.C + c;
+    }
+    st4s(p.g_y, p.g_y_dtype, dst, gy);
+  }
+  float* const accs[3] = {a_next, a_rgb, a_dem};
+  float* const dsts[3] = {p.dot_next, p.dot_rgb, p.dot_demod};
+  for (int k = 0; k < 3; ++k) {
+    if (dsts[k] == nullptr) continue;                  // uniform across the block
+    __syncthreads();
+#pragma unroll
+    for (int j = 0; j < 4; ++j) red[threadIdx.x * 4 + j] = accs[k][j];
+    __syncthreads();
+    if (lane == 0) {
+      float s[4] = {0.f, 0.f, 0.f, 0.f};
+      for (int l = 0; l < lanes; ++l)
+#pragma unroll
+        for (int j = 0; j < 4; ++j) s[j] += red[(l * c4n + cg) * 4 + j];
+      float* d = dsts[k] + (n * p.parts + part) * p.C + c;
+#pragma unroll
+      for (int j = 0; j < 4; ++j) d[j] = s[j];
+    }
+  }
+}
+
+// ds[n][c] = sum_parts dot_mod[n][.][c] - s[n][c] * sum_o (sum_parts dot_demod[n][.][o]) * demod[n][o]^2 * wsq[o][c]
+// (the modulation term and the demodulation adjoint d demod_o / d s_c = -demod_o^3 s_c wsq[o][c]); one block per sample.
+__global__ void __launch_bounds__(256) style_bwd_kernel(const float* __restrict__ dot_mod, int parts_mod, const float* __restrict__ dot_demod,
+                                                        int parts_demod, const float* __restrict__ s, const float* __restrict__ demod,
+                                                        const float* __restrict__ wsq, int cin, int cout, float* __restrict__ ds) {
+  extern __shared__ float q[];                          // [cout]
+  const int64_t n = blockIdx.x;
+  if (dot_demod != nullptr) {
+    for (int o = threadIdx.x; o < cout; o += 256) {
+      float a = 0.f;
+      for (int pp = 0; pp < parts_demod; ++pp) a += dot_demod[(n * parts_demod + pp) * cout + o];
+      const float d = demod[n * cout + o];
+      q[o] = a * d * d;
+    }
+  }
+  __syncthreads();
+  for (int c = threadIdx.x; c < cin; c += 256) {
+    float m = 0.f;
+    if (dot_mod != nullptr)
+      for (int pp = 0; pp < parts_mod; ++pp) m += dot_mod[(n * parts_mod + pp) * cin + c];
+    if (dot_demod != nullptr) {
+      float t = 0.f;
+      for (int o = 0; o < cout; ++o) t = fmaf(q[o], __ldg(wsq + (int64_t)o * cin + c), t);
+      m = fmaf(-s[n * cin + c], t, m);
+    }
+    ds[n * cin + c] = m;
+  }
+}
+
+// adjoint of image_pool_out_kernel: g_o = g_purified * out_scale + g_cls, spread evenly over the k1 x k1 (x k2 x k2) source pixels;
+// masked rows (set to -1 by the forward) pass no gradient.  One thread per generator pixel, float4 store (4th channel = padding, 0).
+__global__ void image_pool_out_bwd_kernel(const float* __restrict__ g_pur, const void* g_cls, int cls_dtype, int N, int S, int k1, int k2,
+                                          int mask_rows, float out_scale, float* __restrict__ g_img) {
+  const int Sp = S / k1, So = Sp / k2;
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;        // over (n, Y, X)
+  if (idx >= (int64_t)N * S * S) return;
+  const int X = (int)(idx % S);
+  const int Y = (int)((idx / S) % S);
+  const int64_t n = idx / ((int64_t)S * S);
+  const int r = Y / k1, q = X / k1;
+  const int y = r / k2, x = q / k2;
+  float g[4] = {0.f, 0.f, 0.f, 0.f};
+  if (!(r < mask_rows || r >= Sp - mask_rows)) {
+    const float inv = 1.f / (float)(k1 * k1 * k2 * k2);
+    for (int c = 0; c < 3; ++c) {
+      float a = 0.f;
+      if (g_pur != nullptr) a = g_pur[((n * 3 + c) * So + y) * So + x] * out_scale;
+      if (g_cls != nullptr) a += ld1s(g_cls, cls_dtype, ((n * So + y) * So + x) * 3 + c);
+      g[c] = a * inv;
+    }
+  }
+  *reinterpret_cast<float4*>(g_img + idx * 4) = make_float4(g[0], g[1], g[2], g[3]);
+}
+
+// adjoint of latent_lerp w.r.t. the codes: g_codes[b,l,:] = (1 - a_l) * g_out[b,l,:]
+__global__ void latent_lerp_bwd_kernel(const float* __restrict__ g_out, const float* __restrict__ alphas, int L, int D, int64_t total,
+                                       float* __restrict__ g_codes) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= total) return;
+  g_codes[i] = (1.f - alphas[(i / D) % L]) * g_out[i];
+}
+
 }  // namespace ga
 
 using namespace ga;
@@ -478,6 +645,89 @@ extern "C" int ga_latent_lerp(const float* codes, const float* styles, const flo
   const int64_t total = (int64_t)b * l * d;
   if (total == 0) return 0;
   latent_lerp_kernel<<<cdiv(total, 256), 256, 0, (cudaStream_t)stream>>>(codes, styles, alphas_dev, l, d, total, out);
+  GA_LAUNCH_OK();
+  return 0;
+}
+
+extern "C" int ga_styled_bias_act_bwd_parts(int hw, int c) {
+  if (hw <= 0 || c <= 0) return 0;
+  const int ppp = sba_bwd_pix_per_part(c);
+  return (hw + ppp - 1) / ppp;
+}
+
+extern "C" int ga_styled_bias_act_bwd(const ga_tensor* v, const ga_tensor* g_next, const float* s_next, const float* g_rgb, const float* w_rgb,
+                                      const float* s_rgb, const float* demod, const float* noise_hw, float noise_w, const float* bias, int phases,
+                                      const ga_tensor* g_y, float* dot_next, float* dot_rgb, float* dot_demod, void* stream) {
+  GA_CHECK(v && (g_next || g_rgb), "ga_styled_bias_act_bwd: null argument");
+  const int C = v->c;
+  GA_CHECK(C % 4 == 0 && C / 4 <= 256 && 256 % (C / 4) == 0, "ga_styled_bias_act_bwd: channels must be 4 * a power of two <= 1024, got %d", C);
+  GA_CHECK(!g_next || same_shape(g_next, v), "ga_styled_bias_act_bwd: g_next must have the activation's shape");
+  GA_CHECK(!g_rgb || (w_rgb && s_rgb), "ga_styled_bias_act_bwd: the RGB branch needs its weights and style");
+  GA_CHECK(!dot_rgb || g_rgb, "ga_styled_bias_act_bwd: dot_rgb needs g_rgb");
+  GA_CHECK(!g_y || demod, "ga_styled_bias_act_bwd: g_y needs demod");
+  GA_CHECK(!dot_demod || g_y, "ga_styled_bias_act_bwd: dot_demod needs g_y");
+  if (g_y) {
+    if (phases) GA_CHECK(v->h % 2 == 0 && v->w % 2 == 0 && g_y->n == v->n && g_y->h * 2 == v->h && g_y->w * 2 == v->w && g_y->c == 4 * C,
+                         "ga_styled_bias_act_bwd: phase gradient must be [n][h/2][w/2][4*c]");
+    else GA_CHECK(same_shape(g_y, v), "ga_styled_bias_act_bwd: g_y shape mismatch");
+  }
+  // 4-channel vectors: 16 bytes in fp32, 8 in bf16
+  auto vec_aligned = [](const ga_tensor* t) { return !t || (((uintptr_t)t->data) % (t->dtype == GA_F32 ? 16 : 8)) == 0; };
+  GA_CHECK(vec_aligned(v) && vec_aligned(g_next) && vec_aligned(g_y) && (((uintptr_t)g_rgb) | ((uintptr_t)w_rgb)) % 16 == 0,
+           "ga_styled_bias_act_bwd: tensors must be aligned to 4 channels (g_rgb / w_rgb to 16 bytes)");
+  const int hw = v->h * v->w;
+  if ((int64_t)v->n * hw == 0) return 0;
+  GA_CHECK(v->n <= 65535, "ga_styled_bias_act_bwd: batch too large");
+  SbaBwd p;
+  p.v = v->data; p.v_dtype = v->dtype;
+  p.g_next = g_next ? g_next->data : nullptr; p.g_next_dtype = g_next ? g_next->dtype : GA_F32; p.s_next = s_next;
+  p.g_rgb = g_rgb; p.w_rgb = g_rgb ? w_rgb : nullptr; p.s_rgb = s_rgb;
+  p.demod = demod; p.noise = noise_hw; p.noise_w = noise_w; p.bias = bias;
+  p.g_y = g_y ? g_y->data : nullptr; p.g_y_dtype = g_y ? g_y->dtype : GA_F32; p.phases = phases;
+  p.dot_next = g_next ? dot_next : nullptr; p.dot_rgb = dot_rgb; p.dot_demod = dot_demod;
+  p.H = v->h; p.W = v->w; p.C = C; p.ppp = sba_bwd_pix_per_part(C); p.parts = ga_styled_bias_act_bwd_parts(hw, C);
+  const size_t smem = (size_t)(p.w_rgb ? C * 4 : 0) * sizeof(float) + 256 * 4 * sizeof(float);
+  GA_CHECK(smem <= 48 * 1024, "ga_styled_bias_act_bwd: too many channels");
+  styled_bias_act_bwd_kernel<<<dim3(p.parts, v->n), 256, smem, (cudaStream_t)stream>>>(p);
+  GA_LAUNCH_OK();
+  return 0;
+}
+
+extern "C" int ga_style_bwd(const float* dot_mod, int parts_mod, const float* dot_demod, int parts_demod, const float* s, const float* demod,
+                            const float* wsq, int n, int cin, int cout, float* ds, void* stream) {
+  GA_CHECK(ds && n >= 0 && cin > 0 && (dot_mod || dot_demod), "ga_style_bwd: bad arguments");
+  GA_CHECK(!dot_mod || parts_mod > 0, "ga_style_bwd: parts_mod must be positive");
+  GA_CHECK(!dot_demod || (parts_demod > 0 && s && demod && wsq && cout > 0), "ga_style_bwd: the demodulation term needs s, demod, wsq, cout");
+  if (n == 0) return 0;
+  const size_t smem = dot_demod ? (size_t)cout * sizeof(float) : 0;
+  GA_CHECK(smem <= 48 * 1024, "ga_style_bwd: too many output channels");
+  style_bwd_kernel<<<n, 256, smem, (cudaStream_t)stream>>>(dot_mod, parts_mod, dot_demod, parts_demod, s, demod, wsq, cin, cout, ds);
+  GA_LAUNCH_OK();
+  return 0;
+}
+
+extern "C" int ga_image_pool_out_bwd(const float* g_purified_nchw, const ga_tensor* g_cls, int k1, int k2, int mask_rows, float out_scale,
+                                     const ga_tensor* g_img, void* stream) {
+  GA_CHECK(g_img && g_img->dtype == GA_F32 && g_img->c == 4 && g_img->h == g_img->w && k1 >= 1 && (k2 == 1 || k2 == 2) &&
+               g_img->h % (k1 * k2) == 0 && mask_rows >= 0 && (g_purified_nchw || g_cls),
+           "ga_image_pool_out_bwd: bad arguments");
+  const int so = g_img->h / (k1 * k2);
+  GA_CHECK(!g_cls || (g_cls->n == g_img->n && g_cls->h == so && g_cls->w == so && g_cls->c == 3), "ga_image_pool_out_bwd: g_cls shape mismatch");
+  GA_CHECK((((uintptr_t)g_img->data) & 15) == 0, "ga_image_pool_out_bwd: g_img must be 16-byte aligned");
+  const int64_t total = numel(g_img) / 4;
+  if (total == 0) return 0;
+  image_pool_out_bwd_kernel<<<cdiv(total, 256), 256, 0, (cudaStream_t)stream>>>(g_purified_nchw, g_cls ? g_cls->data : nullptr,
+                                                                                g_cls ? g_cls->dtype : GA_F32, g_img->n, g_img->h, k1, k2,
+                                                                                mask_rows, out_scale, (float*)g_img->data);
+  GA_LAUNCH_OK();
+  return 0;
+}
+
+extern "C" int ga_latent_lerp_bwd(const float* g_out, const float* alphas_dev, int b, int l, int d, float* g_codes, void* stream) {
+  GA_CHECK(g_out && alphas_dev && g_codes && b >= 0 && l > 0 && d > 0, "ga_latent_lerp_bwd: bad arguments");
+  const int64_t total = (int64_t)b * l * d;
+  if (total == 0) return 0;
+  latent_lerp_bwd_kernel<<<cdiv(total, 256), 256, 0, (cudaStream_t)stream>>>(g_out, alphas_dev, l, d, total, g_codes);
   GA_LAUNCH_OK();
   return 0;
 }

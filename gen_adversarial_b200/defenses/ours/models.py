@@ -178,11 +178,11 @@ class _StyleGanDefenseBase(MLVGMDefenseModel):
                               seed=self._seed_now, sample0=self.sample_offset, normalize=normalize, taps_cache=self._taps_cache)
         return x
 
-    def _decode(self, codes, cls_dtype, want_purified=True, denorm=(0.5, 0.5)):
+    def _decode(self, codes, cls_dtype, want_purified=True, denorm=(0.5, 0.5), tape=None):
         """synthesis in batch chunks + the fused output kernel -> (purified NCHW [0,1], classifier input NHWC)"""
         dec = self.autoencoder.decoder
         dec.max_chunk = self.max_chunk
-        outs = dec.synthesis(codes, sink=lambda img: self._pool_out(img, cls_dtype, want_purified, denorm))
+        outs = dec.synthesis(codes, sink=lambda img: self._pool_out(img, cls_dtype, want_purified, denorm), tape=tape)
         cat = lambda ts: None if ts[0] is None else (ts[0] if len(ts) == 1 else torch.cat(ts, dim=0))
         return cat([o[0] for o in outs]), cat([o[1] for o in outs])
 
@@ -199,11 +199,45 @@ class _StyleGanDefenseBase(MLVGMDefenseModel):
 
     def _forward_cuda(self, batch: torch.Tensor, tape=None):
         if tape is not None:
-            raise NotImplementedError("input-gradient backward through the StyleGAN purifiers is not built (SURVEY 8f rank 3)")
+            raise NotImplementedError("input-gradient backward through the StyleGAN purifiers: the encoder half (image -> codes) is not "
+                                      "built; the decode half is differentiable through from_codes()")
         x = self._preprocessed(batch)
         codes = self._mix(self._encode(x))
         purified, cls_in = self._decode(codes, self.classifier.classifier.adt)
         return self.classifier.classifier.forward(cls_in), purified
+
+    def from_codes(self, codes: torch.Tensor, preds_only: bool = True):
+        """The tail of `__call__` from the encoder's W+ codes (B, n_codes, 512) fp32: mix with the style noise (same seed / explicit-noise /
+        `sample_offset` rules as a call) -> synthesis -> pool -> classifier.  -> logits, or (logits, purified) when not preds_only.
+        Differentiable w.r.t. `codes` (input gradient only; repeated backward through one forward works)."""
+        if codes.requires_grad and torch.is_grad_enabled():
+            from ...autograd import codes_apply
+            preds, purified = codes_apply(self, codes)
+        else:
+            preds, purified = self._from_codes_cuda(codes.detach())
+        return preds if preds_only else (preds, purified)
+
+    def _from_codes_cuda(self, codes: torch.Tensor, tape=None):
+        """-> (logits, purified); tape: an `autograd.CodesTape` to fill for `_from_codes_backward`"""
+        self._seed_now = self._next_seed()
+        alphas = self._alphas_device()
+        latent = self._mix(codes.to(self.autoencoder.device, torch.float32).contiguous())
+        cls_eng = self.classifier.classifier
+        purified, cls_in = self._decode(latent, cls_eng.adt, tape=tape.syn if tape is not None else None)
+        if tape is None:
+            return cls_eng.forward(cls_in), purified
+        tape.alphas = alphas.clone()                     # the caller may reassign interpolation_alphas before a backward
+        return cls_eng.forward(cls_in, tape=tape.cls), purified
+
+    def _from_codes_backward(self, tape, g_preds, g_purified) -> torch.Tensor:
+        """(d loss / d logits | None, d loss / d purified | None) -> d loss / d codes (B, n_codes, 512) fp32"""
+        g_cls = self.classifier.classifier.backward(tape.cls, g_preds.contiguous().to(torch.float32)) if g_preds is not None else None
+        g_pur = g_purified.contiguous().to(torch.float32) if g_purified is not None else None
+        dec = self.autoencoder.decoder
+        g_img = [self._pool_out_bwd(g_pur[lo:lo + n] if g_pur is not None else None, g_cls[lo:lo + n] if g_cls is not None else None,
+                                    dec.size) for lo, n in tape.syn.slices]
+        dec.max_chunk = self.max_chunk
+        return ops.latent_lerp_bwd(dec.synthesis_backward(tape.syn, g_img), tape.alphas)
 
 
 class E4EStyleGanDefenseModel(_StyleGanDefenseBase, torch.nn.Module):
@@ -240,6 +274,9 @@ class E4EStyleGanDefenseModel(_StyleGanDefenseBase, torch.nn.Module):
     def _pool_out(self, img, cls_dtype, want_purified, denorm):
         k = img.shape[1] // 256                                                           # face_pool -> 256 x 256, psp.py:26,114
         return ops.image_pool_out(img, k, 1, 0, denorm, cls_dtype, want_purified)
+
+    def _pool_out_bwd(self, g_pur, g_cls, size):
+        return ops.image_pool_out_bwd(g_pur, g_cls, size, size // 256, 1, 0, 0.5)
 
 
 class TransStyleGanDefenseModel(_StyleGanDefenseBase, torch.nn.Module):
@@ -281,3 +318,6 @@ class TransStyleGanDefenseModel(_StyleGanDefenseBase, torch.nn.Module):
     def _pool_out(self, img, cls_dtype, want_purified, denorm):
         k = img.shape[1] // 256                                                           # face_pool, models.py:346
         return ops.image_pool_out(img, k, 2, 32, denorm, cls_dtype, want_purified)        # rows := -1, resize 256 -> 128 (:347-351)
+
+    def _pool_out_bwd(self, g_pur, g_cls, size):
+        return ops.image_pool_out_bwd(g_pur, g_cls, size, size // 256, 2, 32, 0.5)

@@ -766,5 +766,60 @@ def preprocess_bwd(g_nhwc, pre_nchw, blur: bool, normalize: bool = True, taps_ca
     return gx
 
 
+def styled_bias_act_bwd_parts(hw: int, c: int) -> int:
+    """number of fixed pixel slices of the per-(sample, channel) partial sums of `styled_bias_act_bwd`"""
+    return int(_lib.lib().ga_styled_bias_act_bwd_parts(hw, c))
+
+
+@_timed("styled_bias_act_bwd", hbm=True)
+def styled_bias_act_bwd(v, g_next, s_next, g_rgb, w_rgb, s_rgb, demod, noise_hw, noise_w: float, bias, phases: bool, gy_dtype,
+                        dot_next=None, dot_rgb=None, dot_demod=None, want_gy: bool = True):
+    """backward of one styled layer's epilogue (styled_bias_act + the ToRGB 1x1 conv fed by it), v = the taped activation.
+    -> g_y (conv-output gradient; phase-major [n,h/2,w/2,4c] when `phases`) or None; the dots land in the caller's
+    [n, styled_bias_act_bwd_parts(h*w, c), c] fp32 buffers"""
+    n, h, w, c = v.shape
+    g_y = None
+    if want_gy:
+        g_y = torch.empty((n, h // 2, w // 2, 4 * c) if phases else (n, h, w, c), device=v.device, dtype=gy_dtype)
+    _lib.check(_lib.lib().ga_styled_bias_act_bwd(gt(v), gt(g_next), ptr(s_next), ptr(g_rgb), ptr(w_rgb), ptr(s_rgb), ptr(demod),
+                                                 ptr(noise_hw), float(noise_w), ptr(bias), int(phases), gt(g_y), ptr(dot_next), ptr(dot_rgb),
+                                                 ptr(dot_demod), stream()), "styled_bias_act_bwd")
+    return g_y
+
+
+@_timed("style_bwd")
+def style_bwd(dot_mod, dot_demod, s, demod, wsq) -> torch.Tensor:
+    """d loss / d s (n, cin) of a modulated layer from its partial dots (see `styled_bias_act_bwd`); dot_demod / demod / wsq are None for
+    ToRGB layers (no demodulation)"""
+    n, cin = s.shape
+    cout = wsq.shape[0] if wsq is not None else 0
+    ds = torch.empty((n, cin), device=s.device, dtype=torch.float32)
+    _lib.check(_lib.lib().ga_style_bwd(ptr(dot_mod), dot_mod.shape[1] if dot_mod is not None else 0, ptr(dot_demod),
+                                       dot_demod.shape[1] if dot_demod is not None else 0, ptr(s), ptr(demod), ptr(wsq), n, cin, cout,
+                                       ptr(ds), stream()), "style_bwd")
+    return ds
+
+
+@_timed("image_pool_out_bwd", hbm=True)
+def image_pool_out_bwd(g_purified, g_cls, size: int, k1: int, k2: int = 1, mask_rows: int = 0, out_scale: float = 0.5):
+    """adjoint of `image_pool_out`: (g_purified NCHW fp32 | None, g_cls NHWC | None) -> generator image gradient (n, size, size, 4) fp32"""
+    n = (g_purified if g_purified is not None else g_cls).shape[0]
+    g_img = torch.empty((n, size, size, 4), device=(g_purified if g_purified is not None else g_cls).device, dtype=torch.float32)
+    _lib.check(_lib.lib().ga_image_pool_out_bwd(ptr(g_purified.contiguous()) if g_purified is not None else None,
+                                                gt(g_cls.contiguous()) if g_cls is not None else None, k1, k2, mask_rows, float(out_scale),
+                                                gt(g_img), stream()), "image_pool_out_bwd")
+    return g_img
+
+
+@_timed("latent_lerp_bwd")
+def latent_lerp_bwd(g_out, alphas_dev):
+    """adjoint of `latent_lerp` w.r.t. the codes: (1 - alpha_l) * g_out[:, l]"""
+    b, l, d = g_out.shape
+    g_out = g_out.contiguous()
+    out = torch.empty_like(g_out)
+    _lib.check(_lib.lib().ga_latent_lerp_bwd(ptr(g_out), ptr(alphas_dev), b, l, d, ptr(out), stream()), "latent_lerp_bwd")
+    return out
+
+
 def launch_count(reset: bool = False) -> int:
     return int(_lib.lib().ga_launch_count(int(reset)))

@@ -47,11 +47,25 @@ def superpixel_weights(w: torch.Tensor) -> torch.Tensor:
 
 
 class _Styled:
-    __slots__ = ("mod", "conv", "conv_sp", "phase_convs", "wsq", "noise", "noise_w", "bias", "up", "cin", "cout")
+    __slots__ = ("mod", "conv", "conv_sp", "phase_convs", "wsq", "noise", "noise_w", "bias", "up", "cin", "cout",
+                 "mod_d", "conv_d", "conv_sp_d", "phase_d")
 
 
 class _ToRGB:
-    __slots__ = ("mod", "conv", "bias", "up_kernel")
+    __slots__ = ("mod", "conv", "bias", "up_kernel", "mod_d", "up_kernel_d")
+
+
+class SynthesisTape:
+    """what `StyleGan2Engine.synthesis(..., tape=...)` leaves for `synthesis_backward`: the styles / demodulation factors of the whole
+    batch, every styled layer's activation act(pre) per batch slice (as the forward produced it: fp32 up to `f32_conv_out_res`, the
+    mode's activation dtype above) and the output slices in forward order"""
+
+    def __init__(self):
+        self.batch = 0
+        self.n_codes = 0
+        self.st = None
+        self.acts = {}          # (id(layer), first sample of the slice) -> activation
+        self.slices = []        # (first sample, size) of each output slice
 
 
 class StyleGan2Engine:
@@ -87,6 +101,7 @@ class StyleGan2Engine:
                                 self._fold_rgb(f, f"to_rgbs.{j}", up=True)))
         num_layers = (self.log_size - 2) * 2 + 1
         self.noises = [f.dev32(f.f64(f"noises.noise_{i}")[0, 0]) for i in range(num_layers)]
+        self._has_adjoint = False
 
     # ------------------------------------------------------------------ load-time folds
     def _fold_mod(self, f: Folder, prefix: str):
@@ -190,7 +205,7 @@ class StyleGan2Engine:
             out[id(layer)] = (st, ops.style_demod(st, layer.wsq) if kind == "styled" else None)
         return out
 
-    def _styled(self, xs, s: _Styled, demod, noise, scale_next, scale_rgb):
+    def _styled(self, xs, s: _Styled, demod, noise, scale_next, scale_rgb, tape=None, key=None):
         """xs: input already scaled by this layer's style.  -> (act * scale_next | None, act * scale_rgb | None): the output is
         handed to its consumers pre-modulated (the fused epilogue kernel applies their style vectors on the fp32 value)"""
         # conv outputs at <= 128^2 stay fp32 until the fused epilogue (one bf16 rounding less per layer where it is almost free:
@@ -208,7 +223,15 @@ class StyleGan2Engine:
             phases = True
         r = ops.styled_bias_act(y, phases, demod, noise, s.noise_w, s.bias, ACT_LRELU_SQRT2, None, self.adt, scale_a=scale_next,
                                 scale_b=scale_rgb, want_out=scale_next is not None)
+        if tape is not None:
+            # the unmodulated activation for the backward: a second pass of the same epilogue, so the values handed to the consumers are
+            # exactly those of an untaped forward
+            tape.acts[(id(s), key)] = ops.styled_bias_act(y, phases, demod, noise, s.noise_w, s.bias, ACT_LRELU_SQRT2, None,
+                                                          self._tape_dtype(h * (2 if s.up else 1)))
         return r if scale_rgb is not None else (r, None)
+
+    def _tape_dtype(self, res: int):
+        return torch.float32 if (not self.bf16 or res <= self.f32_conv_out_res) else self.adt
 
     fuse_rgb = __import__("os").environ.get("GA_SG_FUSE_RGB", "1") != "0"
 
@@ -228,46 +251,155 @@ class StyleGan2Engine:
         cout = self.blocks[j][0].cout
         return max(1, (1 << 29) // (res * res * cout))
 
-    def _run_blocks(self, j, x, skip, st, lo, sink, outs):
+    def _run_blocks(self, j, x, skip, st, lo, sink, outs, tape=None):
         """blocks j.. on samples [lo, lo + n): low resolutions run on the whole batch, high resolutions on slices (recursive split)"""
         n = skip.shape[0]
         if j == len(self.blocks):
+            if tape is not None:
+                tape.slices.append((lo, n))
             outs.append(sink(skip) if sink is not None else skip)
             return
         cap = self.max_chunk or self._cap(j)
         if n > cap:
             for o in range(0, n, cap):
-                self._run_blocks(j, x[o:o + cap], skip[o:o + cap], st, lo + o, sink, outs)
+                self._run_blocks(j, x[o:o + cap], skip[o:o + cap], st, lo + o, sink, outs, tape)
             return
         up, conv, rgb = self.blocks[j]
         sl = slice(lo, lo + n)
         s_conv, d_conv = st[id(conv)]
         s_rgb, _ = st[id(rgb)]
         s_next = st[id(self.blocks[j + 1][0])][0][sl] if j + 1 < len(self.blocks) else None
-        x, _ = self._styled(x, up, st[id(up)][1][sl], self.noises[2 * j + 1], s_conv[sl], None)
-        x, xr = self._styled(x, conv, d_conv[sl], self.noises[2 * j + 2], s_next, s_rgb[sl])
+        x, _ = self._styled(x, up, st[id(up)][1][sl], self.noises[2 * j + 1], s_conv[sl], None, tape, lo)
+        x, xr = self._styled(x, conv, d_conv[sl], self.noises[2 * j + 2], s_next, s_rgb[sl], tape, lo)
         skip = self._rgb(xr, rgb, skip)
-        self._run_blocks(j + 1, x, skip, st, lo, sink, outs)
+        self._run_blocks(j + 1, x, skip, st, lo, sink, outs, tape)
 
     max_chunk = None
     superpixel = __import__("os").environ.get("GA_SG_SUPERPIXEL", "1") != "0"
     f32_conv_out_res = int(__import__("os").environ.get("GA_SG_F32_RES", "128"))
 
-    def synthesis(self, latent: torch.Tensor, sink=None):
+    def synthesis(self, latent: torch.Tensor, sink=None, tape: Optional[SynthesisTape] = None):
         """latent: (B, >= n_latent, style_dim) fp32 -> list of RGB image slices NHWC (n_i, size, size, 4) fp32 in batch order (4th
-        channel is padding), or of `sink(slice)` results when a sink is given (the caller pools each slice as soon as it exists)"""
+        channel is padding), or of `sink(slice)` results when a sink is given (the caller pools each slice as soon as it exists).
+        tape: a fresh `SynthesisTape` that records what `synthesis_backward` needs (the outputs do not change)."""
         b = latent.shape[0]
         assert latent.shape[1] >= self.n_latent, (latent.shape, self.n_latent)
         latent = latent.to(torch.float32)
         st = self._styles(latent)
+        if tape is not None:
+            tape.batch, tape.n_codes, tape.st = b, latent.shape[1], st
         s1, d1 = st[id(self.conv1)]
         x0 = ops.channel_scale(self.const_input.expand(b, -1, -1, -1).contiguous(), s1, self.adt)
         s_next = st[id(self.blocks[0][0])][0] if self.blocks else None
-        x, xr = self._styled(x0, self.conv1, d1, self.noises[0], s_next, st[id(self.to_rgb1)][0])
+        x, xr = self._styled(x0, self.conv1, d1, self.noises[0], s_next, st[id(self.to_rgb1)][0], tape, 0)
         skip = self._rgb(xr, self.to_rgb1, None)
         outs = []
-        self._run_blocks(0, x, skip, st, 0, sink, outs)
+        self._run_blocks(0, x, skip, st, 0, sink, outs, tape)
         return outs
+
+    # ------------------------------------------------------------------ input-gradient backward (W+ codes; weights frozen)
+    def _build_adjoint(self):
+        """flipped / transposed weights of every conv, folded in fp64 on the first backward (forward-only use pays nothing):
+        3x3 convs -> their dgrad conv (the superpixel pair conv of the 32-channel layers -> superpixel_weights of the adjoint, which IS the
+        adjoint of the pair conv), the up-sampling phase conv -> ONE 3x3 conv over the de-interleaved [h, w, 4 cout] gradient, modulation
+        EqualLinears -> their transposes (fp32 SIMT), ToRGB skip up-sampling -> the flipped FIR (down 2)"""
+        from .nvae_engine import make_dgrad_layer
+        f = Folder({}, self.device, want_tc=self.bf16)
+        f32 = Folder({}, self.device, want_tc=False)
+        for kind, layer, _ in self._plan():
+            layer.mod_d = make_dgrad_layer(f32, layer.mod, False)
+            if kind == "rgb":
+                layer.up_kernel_d = layer.up_kernel.flip(0, 1).contiguous() if layer.up_kernel is not None else None
+                continue
+            if layer.up:
+                layer.phase_d = make_dgrad_layer(f, layer.phase_convs, self.bf16)
+                layer.conv_d = layer.conv_sp_d = None
+            else:
+                layer.phase_d = None
+                layer.conv_d = make_dgrad_layer(f, layer.conv, self.bf16)
+                layer.conv_sp_d = None
+                if layer.conv_sp is not None:
+                    wt = layer.conv_d.w_simt.detach().to("cpu", torch.float64).view(3, 3, layer.cout, layer.cin).permute(3, 2, 0, 1)
+                    layer.conv_sp_d = f.conv(superpixel_weights(wt), None, pad=1, name=layer.conv.name + ".dgrad.superpixel", simt=False)
+        self._has_adjoint = True
+
+    def _dgrad(self, s: _Styled, g, f32: bool):
+        """gradient w.r.t. the layer's modulated input from the conv-output gradient g (de-interleaved phases for up-sampling layers)"""
+        if s.up:
+            return self._conv(g, s.phase_d, want_f32=f32)
+        b, h, w, _ = g.shape
+        if s.conv_sp_d is not None and not f32 and g.dtype == torch.bfloat16 and w % 2 == 0 and g.is_contiguous():
+            return self._conv(g.view(b, h, w // 2, 2 * s.cout), s.conv_sp_d).view(b, h, w, s.cin)
+        return self._conv(g, s.conv_d, want_f32=f32)
+
+    def _layer_bwd(self, s: _Styled, tape, lo, n, g_next, nxt, rgb, g_rgb, noise, dots):
+        """one styled layer on samples [lo, lo + n): epilogue adjoint (+ partial dots) then the conv's dgrad -> gradient w.r.t. its
+        modulated input"""
+        st, sl = tape.st, slice(lo, lo + n)
+        v = tape.acts[(id(s), lo)]
+        hw, c = v.shape[1] * v.shape[2], v.shape[3]
+        f32 = not self.bf16 or v.shape[1] // (2 if s.up else 1) <= self.f32_conv_out_res
+        g_y = ops.styled_bias_act_bwd(
+            v, g_next, st[id(nxt)][0][sl] if nxt is not None else None, g_rgb, rgb.conv.w_simt if rgb is not None else None,
+            st[id(rgb)][0][sl] if rgb is not None else None, st[id(s)][1][sl], noise, s.noise_w, s.bias, s.up,
+            torch.bfloat16 if self.bf16 else torch.float32,
+            dot_next=dots(nxt, "mod", hw, c)[sl] if nxt is not None else None,
+            dot_rgb=dots(rgb, "mod", hw, c)[sl] if rgb is not None else None,
+            dot_demod=dots(s, "demod", hw, c)[sl])
+        return self._dgrad(s, g_y, f32)
+
+    def _bwd_blocks(self, j, lo, n, tape, g_it, dots):
+        """reverse of `_run_blocks` on samples [lo, lo + n) -> (gradient w.r.t. the modulated input of block j's up-sampling conv,
+        gradient w.r.t. the RGB skip entering block j)"""
+        if j == len(self.blocks):
+            g = next(g_it)
+            if tuple(g.shape) != (n, self.size, self.size, 4):
+                raise ValueError(f"image gradient slice must have shape {(n, self.size, self.size, 4)}, got {tuple(g.shape)}")
+            return None, g.to(torch.float32).contiguous()
+        cap = self.max_chunk or self._cap(j)
+        if n > cap:
+            parts = [self._bwd_blocks(j, lo + o, min(cap, n - o), tape, g_it, dots) for o in range(0, n, cap)]
+            return torch.cat([p[0] for p in parts], dim=0), torch.cat([p[1] for p in parts], dim=0)
+        up, conv, rgb = self.blocks[j]
+        nxt = self.blocks[j + 1][0] if j + 1 < len(self.blocks) else None
+        g_next, g_skip = self._bwd_blocks(j + 1, lo, n, tape, g_it, dots)
+        g_x = self._layer_bwd(conv, tape, lo, n, g_next, nxt, rgb, g_skip, self.noises[2 * j + 2], dots)
+        g_x = self._layer_bwd(up, tape, lo, n, g_x, conv, None, None, self.noises[2 * j + 1], dots)
+        # adjoint of the skip's Upsample (upfirdn2d up 2, pad (2, 1)): the flipped FIR, down 2, pad (1, 1)
+        return g_x, ops.upfirdn2d(g_skip, rgb.up_kernel_d, up=1, down=2, pad=(1, 1))
+
+    def synthesis_backward(self, tape: SynthesisTape, g_slices) -> torch.Tensor:
+        """input gradient of `synthesis`: g_slices = gradients of the output image slices (n_i, size, size, 4) fp32 in the forward's slice
+        order -> gradient w.r.t. the latent (B, n_codes, style_dim) fp32.  The tape is only read: any number of backward passes work."""
+        if not self._has_adjoint:
+            self._build_adjoint()
+        b, st = tape.batch, tape.st
+        bufs = {}
+
+        def dots(layer, kind, hw, c):
+            key = (id(layer), kind)
+            if key not in bufs:
+                bufs[key] = torch.empty((b, ops.styled_bias_act_bwd_parts(hw, c), c), device=self.device, dtype=torch.float32)
+            return bufs[key]
+
+        g_it = iter(g_slices)
+        nxt = self.blocks[0][0] if self.blocks else None
+        g_x, g_skip = self._bwd_blocks(0, 0, b, tape, g_it, dots)
+        g_x = self._layer_bwd(self.conv1, tape, 0, b, g_x, nxt, self.to_rgb1, g_skip, self.noises[0], dots)
+        # conv1's modulation acts on the constant input: its dot is the only thing left to form there
+        const = self.const_input.expand(b, -1, -1, -1).contiguous()
+        ops.styled_bias_act_bwd(const, g_x, None, None, None, None, None, None, 0.0, None, False, None, want_gy=False,
+                                dot_next=dots(self.conv1, "mod", 16, const.shape[3]))
+        g_lat = [None] * self.n_latent
+        for kind, layer, idx in self._plan():
+            s, demod = st[id(layer)]
+            ds = ops.style_bwd(bufs[(id(layer), "mod")], bufs.get((id(layer), "demod")), s, demod, layer.wsq if kind == "styled" else None)
+            # several layers share a latent index: the modulation EqualLinear's adjoint accumulates through the SIMT conv's add epilogue
+            g_lat[idx] = ops.conv2d_simt(ds.view(b, 1, 1, -1), layer.mod_d, torch.float32, add=g_lat[idx])
+        g = torch.cat([t.view(b, 1, self.style_dim) for t in g_lat], dim=1)
+        if tape.n_codes > self.n_latent:
+            g = torch.cat([g, g.new_zeros((b, tape.n_codes - self.n_latent, self.style_dim))], dim=1)
+        return g
 
     def decode(self, latent: torch.Tensor, pool: int = 1, chunk: Optional[int] = None) -> torch.Tensor:
         """`pSp.decode` (psp.py:109-115): synthesis + face_pool (k x k mean) -> NCHW fp32 (B,3,size/pool,size/pool)."""

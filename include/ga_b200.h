@@ -240,6 +240,25 @@ int ga_upfirdn2d(const ga_tensor* in, const float* kernel, int kh, int kw, int u
 int ga_avgpool_to_nchw(const ga_tensor* in, int k, int out_c, float* out_nchw, void* stream);           /* face_pool, psp.py:26,114 */
 int ga_latent_lerp(const float* codes, const float* styles, const float* alphas_dev, int b, int l, int d, float* out,
                    void* stream);                                                                         /* models.py:123-124,338-339 */
+/* ---- input gradient of the W+ decode (codes -> generator -> pooled image), dgrad only.  Per-(sample, channel) sums are written as
+ * partials over fixed pixel slices, [n][parts][c] with parts = ga_styled_bias_act_bwd_parts(h*w, c): no atomics, the same order for a
+ * sample wherever it sits in the batch.
+ * Mirror of ga_styled_bias_act (+ the ToRGB 1x1 adjoint) for one styled layer, v = its taped activation act(pre) [n][h][w][c]:
+ *   g_v = s_next * g_next + s_rgb * (w_rgb^T g_rgb),  g_y = g_v * lrelu'(pre) * sqrt(2) * demod  (phases=1: [n][h/2][w/2][4c], phase-major),
+ *   dot_next += g_next * v,  dot_rgb += (w_rgb^T g_rgb) * v,  dot_demod += g_pre * (pre - bias - noise_w * noise) = demod * d demod.
+ * g_next [n][h][w][c] fp32/bf16 or NULL; g_rgb fp32 [n][h][w][4] with w_rgb fp32 [c][4], s_rgb [n][c], or NULL; g_y NULL: dots only.
+ * c = 4 * a power of two <= 1024. */
+int ga_styled_bias_act_bwd_parts(int hw, int c);
+int ga_styled_bias_act_bwd(const ga_tensor* v, const ga_tensor* g_next /*nullable*/, const float* s_next /*nullable*/,
+                           const float* g_rgb /*nullable*/, const float* w_rgb, const float* s_rgb, const float* demod, const float* noise_hw,
+                           float noise_w, const float* bias, int phases, const ga_tensor* g_y /*nullable*/, float* dot_next /*nullable*/,
+                           float* dot_rgb /*nullable*/, float* dot_demod /*nullable*/, void* stream);
+/* style adjoint: ds[n][c] = sum_parts dot_mod[n][.][c] - s[n][c] * sum_o (sum_parts dot_demod[n][.][o]) demod[n][o]^2 wsq[o][c]
+ * (modulation term + d demod / d s, generator.py:164-171); either dot array may be NULL */
+int ga_style_bwd(const float* dot_mod, int parts_mod, const float* dot_demod, int parts_demod, const float* s, const float* demod,
+                 const float* wsq, int n, int cin, int cout, float* ds, void* stream);
+/* adjoint of ga_latent_lerp w.r.t. the codes: g_codes[b][l] = (1 - alphas[l]) * g_out[b][l] */
+int ga_latent_lerp_bwd(const float* g_out, const float* alphas_dev, int b, int l, int d, float* g_codes, void* stream);
 
 /* ================================================================ encoder-side pieces of the StyleGAN purifiers (encoders.cu)
  * out (and optional second copy out2) = LayerNorm(x + y) * gamma + beta over the channel dim   transformer.py:54-66 (norm1-3) */
@@ -263,6 +282,10 @@ int ga_resize_bilinear(const ga_tensor* in, int full_h, int crop_y0, const ga_te
  * (psp.py:26,114; models.py:346-351; abstract_models.py:184-185) */
 int ga_image_pool_out(const ga_tensor* in, int k1, int k2, int mask_rows, float out_scale, float out_shift, float* purified_nchw,
                       const ga_tensor* cls_nhwc /*nullable*/, void* stream);
+/* adjoint of ga_image_pool_out: g_img (N,S,S,4) fp32 = pooling adjoint of (g_purified * out_scale + g_cls); masked rows get zero,
+ * the 4th (padding) channel is zero.  g_purified_nchw (N,3,So,So) fp32 and g_cls (N,So,So,3) may each be NULL. */
+int ga_image_pool_out_bwd(const float* g_purified_nchw /*nullable*/, const ga_tensor* g_cls /*nullable*/, int k1, int k2, int mask_rows,
+                          float out_scale, const ga_tensor* g_img, void* stream);
 /* out[l][b][d] ~ N(0, std^2), Philox stream keyed by (seed, l, global sample index): torch.normal(0, std, (n_codes, b, d)), models.py:119,334 */
 int ga_philox_codes(uint64_t seed, int64_t sample0, float std_, int l, int b, int d, float* out, void* stream);
 
