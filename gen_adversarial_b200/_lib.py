@@ -151,6 +151,8 @@ _PROTOS = {
     "ga_image_pool_out": (c_int, [T, c_int, c_int, c_int, c_float, c_float, c_void_p, T, c_void_p]),
     "ga_philox_codes": (c_int, [c_uint64, c_int64, c_float, c_int, c_int, c_int, c_void_p, c_void_p]),
     "ga_latent_mix_fwd": (c_int, [T, T, c_void_p, c_uint64, c_int, c_int64, c_void_p, c_float, c_int, T, c_void_p]),
+    "ga_latent_level": (c_int, [T, T, T, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_uint64, c_int, c_int64, c_void_p,
+                                c_float, c_int, T, T, T, c_void_p]),
     "ga_discmix_mean_fwd": (c_int, [T, c_int, c_void_p, T, c_void_p]),
     "ga_upsample_nearest2x": (c_int, [T, T, c_void_p]),
     "ga_upsample_bilinear2x": (c_int, [T, T, c_void_p]),

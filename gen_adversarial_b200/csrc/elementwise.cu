@@ -23,10 +23,6 @@ __device__ __forceinline__ void st1d(void* base, int dtype, int64_t off, float v
   else reinterpret_cast<__nv_bfloat16*>(base)[off] = __float2bfloat16_rn(v);
 }
 
-__host__ __device__ __forceinline__ uint64_t noise_stream(int64_t sample, int level) {
-  return (uint64_t)sample * 64ull + (uint64_t)level;
-}
-
 // ============================================================================ noise L2 norm pre-pass
 // block-level deterministic sum: warp shuffle tree, then warp 0 adds the per-warp values in fixed order
 __device__ __forceinline__ float block_sum_256(float v) {
@@ -656,7 +652,7 @@ __global__ void __launch_bounds__(128) latent_mix_kernel(const void* __restrict_
                      a * (5.f * tanh_approx(0.2f * mp[u]) + ee[u] * (temp * __expf(5.f * tanh_approx(0.2f * lp[u]))));
         } else {
           if (pp == nullptr) out = (1.f - a) * softclamp5_(mq[u]) + a * (ee[u] * temp);
-          else out = (1.f - a) * softclamp5_(mp[u] + mq[u]) + a * (softclamp5_(mp[u]) + ee[u] * (temp * expf(softclamp5_(lp[u]))));
+          else out = latent_mix_prior(a, mq[u], mp[u], lp[u], ee[u], temp);
         }
       }
       st1d(zout, z_dtype, pix * Cz + zc, out);
@@ -703,7 +699,7 @@ __global__ void __launch_bounds__(256) latent_mix_vec4_kernel(const void* __rest
                       a * (5.f * tanh_approx(0.2f * mp[u]) + ee[u] * (temp * __expf(5.f * tanh_approx(0.2f * lp[u]))));
       } else {
         if (pp == nullptr) out[u] = (1.f - a) * softclamp5_(mq[u]) + a * (ee[u] * temp);
-        else out[u] = (1.f - a) * softclamp5_(mp[u] + mq[u]) + a * (softclamp5_(mp[u]) + ee[u] * (temp * expf(softclamp5_(lp[u]))));
+        else out[u] = latent_mix_prior(a, mq[u], mp[u], lp[u], ee[u], temp);
       }
     }
   }

@@ -49,6 +49,12 @@ __device__ __forceinline__ float sigmoidf_(float x) { return 1.0f / (1.0f + expf
 __device__ __forceinline__ float siluf_(float x) { return x / (1.0f + expf(-x)); }
 __device__ __forceinline__ float eluf_(float x) { return x > 0.0f ? x : expm1f(x); }
 __device__ __forceinline__ float softclamp5_(float x) { return 5.0f * tanhf(x * 0.2f); }
+// one latent channel of a level with a prior (models.py:198-206,243-250):
+//   z = (1-a) * sc(mu_p + mu_q) + a * (sc(mu_p) + eps * T * exp(sc(logsig_p)))
+// shared by latent_mix (elementwise.cu) and the fused level tail (latent_level.cu) so both round identically
+__device__ __forceinline__ float latent_mix_prior(float a, float mq, float mp, float lp, float e, float temp) {
+  return (1.f - a) * softclamp5_(mp + mq) + a * (softclamp5_(mp) + e * (temp * expf(softclamp5_(lp))));
+}
 
 __device__ __forceinline__ float apply_act(float v, int act) {
   switch (act) {
@@ -328,6 +334,10 @@ __device__ __forceinline__ void philox_normal4(uint64_t seed, uint64_t stream, u
   __sincosf(6.283185307179586f * u1, &s0, &c0);
   __sincosf(6.283185307179586f * u3, &s1, &c1);
   z[0] = m0 * c0; z[1] = m0 * s0; z[2] = m1 * c1; z[3] = m1 * s1;
+}
+// Philox stream id of (global sample, level slot): slot 0 is the input noise, slot L + 1 the latent noise of level L
+__host__ __device__ __forceinline__ uint64_t noise_stream(int64_t sample, int level) {
+  return (uint64_t)sample * 64ull + (uint64_t)level;
 }
 // per-level latent noise eps[zc][hw] of one sample (stream = (global sample, level)): the four channels 4j .. 4j+3 of pixel hw are
 // ONE Philox block (counter j * HW + hw), so a thread that owns a pixel draws 4 channels per block with no redundant rounds

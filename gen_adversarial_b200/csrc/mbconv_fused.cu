@@ -57,9 +57,6 @@ struct MbParams {
   unsigned long long* trace;    // debug (ga_debug_mbconv_trace): clock64 stamps [cta < 8][warp 13][chunk 24][event 8]
 };
 
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
 // mbarrier wait for the SIMT warps: back off between polls so that a waiting warp does not take issue slots from the warps of the
 // other role that share its scheduler (activation and depthwise warps wait for each other by design)
 __device__ __forceinline__ void mbar_wait_backoff(uint64_t* bar, uint32_t parity, uint32_t ns = 100) {

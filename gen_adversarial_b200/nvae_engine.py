@@ -89,6 +89,8 @@ class NvaeEngine:
         self.fuse_csum = __import__("os").environ.get("GA_FUSE_CSUM", "1") != "0"     # SE channel sums from the encoder conv2 epilogue
         self.fuse_tape = __import__("os").environ.get("GA_FUSE_TAPE", "1") != "0"     # attack path: taping forward of the decoder cells in the fused kernel
         self.fuse_bwd = int(__import__("os").environ.get("GA_FUSE_BWD", "2"))         # attack path: backward of the decoder cells in the fused kernel
+        # level tail (sampler -> latent mix -> combiner) in one kernel; tests/emu_ops.py emulates the unfused ops only
+        self.fuse_level = __import__("os").environ.get("GA_FUSE_LEVEL", "1") != "0" and not _host_logic_test
         f = Folder(state_dict, self.device, want_tc=self.bf16)
         self._fold(f)
         self._prior_cache = {}
@@ -450,14 +452,21 @@ class NvaeEngine:
                     x_elu = self._elu_copy
                 comb, _ = self._conv(xa, L["enc_comb"], add=stash[(L["s"], L["g"])])
                 _, muq = self._conv(comb, L["enc_sampler"], want_act=False, want_f32=True)
-                pp = self._conv_preact(x32, x_elu, L["dec_sampler"])
                 eps = eps_levels[idx] if eps_levels is not None else None
-                z = ops.latent_mix(muq, pp, eps, seed, idx, sample0, alphas_dev[idx:idx + 1], self.temperature, spec.z, self.zc,
-                                   self.adt)
-                self._tap(f"z{idx}", z[..., :spec.z])
+                if (self.fuse_level and self.bf16 and self.taps is None
+                        and ops.latent_level_supported(x_elu, xa, L["dec_sampler"], L["dec_comb"], spec.z)):
+                    # prior sampler -> latent mix -> combiner in one kernel: pp and z stay on chip (pp is written only for the tape)
+                    xa2, x32_2, pp = ops.latent_level(x_elu, xa, muq, eps, L["dec_sampler"], L["dec_comb"], seed, idx, sample0,
+                                                      alphas_dev[idx:idx + 1], self.temperature, spec.z, want_pp=rec is not None)
+                else:
+                    pp = self._conv_preact(x32, x_elu, L["dec_sampler"])
+                    z = ops.latent_mix(muq, pp, eps, seed, idx, sample0, alphas_dev[idx:idx + 1], self.temperature, spec.z, self.zc,
+                                       self.adt)
+                    self._tap(f"z{idx}", z[..., :spec.z])
+                    xa2, x32_2 = self._conv(xa, L["dec_comb"], want_act=True, want_f32=True, x2=z, aux=L["dec_comb_z"])
                 if rec is not None:
                     rec.append(("level", L, x32, muq, pp, eps, seed, idx, sample0, alphas_dev[idx:idx + 1]))
-                xa, x32 = self._conv(xa, L["dec_comb"], want_act=True, want_f32=True, x2=z, aux=L["dec_comb_z"])
+                xa, x32 = xa2, x32_2
                 idx += 1
             if s in self.up_cells:
                 x32, xa = self._dec_cell(x32, xa, self.up_cells[s], rec)

@@ -331,6 +331,31 @@ def latent_mix(q, p, eps_nchw, seed: int, level: int, sample0: int, alpha_dev, t
     return z
 
 
+def latent_level_supported(x_elu: torch.Tensor, xa: torch.Tensor, sampler: ConvLayer, comb: ConvLayer, zdim: int) -> bool:
+    """can `latent_level` run this level (bf16 tensors, C in {64, 128, 256}, zdim a multiple of 4 up to 32)?"""
+    c = xa.shape[3]
+    return (x_elu is not None and x_elu.dtype == torch.bfloat16 and xa.dtype == torch.bfloat16 and x_elu.shape == xa.shape
+            and c in (64, 128, 256) and zdim % 4 == 0 and 4 <= zdim <= 32 and sampler.w_tc is not None and sampler.cout == 2 * zdim
+            and sampler.kh == 1 and comb.w_tc is not None and comb.kh == 1 and comb.cin == c and comb.cout == c
+            and zdim <= comb.cin2 <= 32 and sampler.bias is not None and comb.bias is not None)
+
+
+@_timed("latent_level", hbm=True)
+def latent_level(x_elu, xa, muq, eps_nchw, sampler: ConvLayer, comb: ConvLayer, seed: int, level: int, sample0: int, alpha_dev,
+                 temperature: float, zdim: int, want_pp: bool = False):
+    """tail of a decoder latent level in one kernel: pp = sampler(x_elu), z = latent_mix(muq, pp, eps), comb([xa | z]).
+    x_elu: ELU(x) in bf16 (the sampler's pre-activated input); comb: the combiner layer with its z weights folded in (cin2 = zc).
+    -> (out bf16, out fp32, pp fp32 | None);  pp only with want_pp (taping forward)"""
+    n, h, w, c = xa.shape
+    ob = torch.empty((n, h, w, c), device=xa.device, dtype=torch.bfloat16)
+    of = torch.empty((n, h, w, c), device=xa.device, dtype=torch.float32)
+    pp = torch.empty((n, h, w, 2 * zdim), device=xa.device, dtype=torch.float32) if want_pp else None
+    _lib.check(_lib.lib().ga_latent_level(gt(x_elu), gt(xa), gt(muq), ptr(eps_nchw), sampler.w_tc.data_ptr(), ptr(sampler.bias),
+                                          comb.w_tc.data_ptr(), ptr(comb.bias), comb.cin2, seed, level, sample0, ptr(alpha_dev),
+                                          temperature, zdim, gt(ob), gt(of), gt(pp), stream()), "latent_level")
+    return ob, of, pp
+
+
 @_timed("discmix_mean", hbm=True)
 def discmix_mean(logits, n_mix: int, cls_dtype=None):
     n, h, w, _ = logits.shape

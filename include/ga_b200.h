@@ -179,6 +179,17 @@ int ga_latent_mix_fwd(const ga_tensor* q, const ga_tensor* p /*nullable*/, const
                       int level, int64_t sample0, const float* alpha_dev /*device scalar*/, float temperature,
                       int zdim, const ga_tensor* z_out, void* stream);
 
+/* ---- tail of a decoder latent level with a prior (NVAE/model.py:226-256), bf16 mode, one tensor-core kernel:
+ *      pp = dec_sampler(x_elu) (+ b_sampler), z = latent mix of (muq, pp, eps) as ga_latent_mix_fwd computes it (level = its `level`),
+ *      out = dec_comb([xa | z]) (+ b_comb) -> out_f32 and out_bf16.  x_elu = ELU(x) and xa: bf16 NHWC with C in {64, 128, 256}; muq: fp32
+ *      NHWC (first zdim channels); w_sampler: bf16 [2*zdim][C]; w_comb: bf16 [C][C + zc] (x weights, then z weights zero-padded to zc
+ *      <= 32 channels); pp_out (nullable, taping): fp32 NHWC [2*zdim].  Bit-identical to dec_sampler conv -> ga_latent_mix_fwd -> combiner
+ *      conv on the tensor-core kernels. */
+int ga_latent_level(const ga_tensor* x_elu, const ga_tensor* xa, const ga_tensor* muq, const float* eps_nchw /*nullable*/,
+                    const void* w_sampler, const float* b_sampler, const void* w_comb, const float* b_comb, int zc, uint64_t seed,
+                    int level, int64_t sample0, const float* alpha_dev /*device scalar*/, float temperature, int zdim,
+                    const ga_tensor* out_bf16, const ga_tensor* out_f32, const ga_tensor* pp_out /*nullable*/, void* stream);
+
 /* ---- DiscMixLogistic(...).mean() + de-normalisation (distributions.py:103-129,231-254; models.py:269-274)
  *      logits NHWC [n][h][w][10*n_mix] -> purified NCHW fp32 in [0,1] (+ optional NHWC classifier input
  *      (p-0.5)/0.5, abstract_models.py:59-60). */

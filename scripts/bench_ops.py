@@ -1,5 +1,5 @@
 """CUDA-event timing of single ops at the attack-path / purify-path shapes (isolated, L2-flushed between launches):
-python scripts/bench_ops.py [dwconv] [k1] [se]"""
+python scripts/bench_ops.py [dwconv] [mbconv] [k1] [hbm] [level]"""
 import sys
 import torch
 sys.path.insert(0, ".")
@@ -179,6 +179,45 @@ def hbm():
         del r, skip, go
 
 
+def level():
+    """tail of one decoder latent level at batch 512, per level size: the three launches (sampler 1x1 -> latent_mix -> combiner 1x1 with z as
+    second source) against the fused latent_level kernel.  GB/s on the fused pass's compulsory bytes (x_elu and xa bf16, muq fp32 in; the
+    stream fp32 + bf16 out), against a device-to-device copy timed in the same process."""
+    import math
+    g = torch.Generator(device=DEV).manual_seed(0)
+    src = torch.empty(1 << 30, dtype=torch.uint8, device=DEV)
+    dst = torch.empty_like(src)
+    peak = 2 * src.numel() / timeit(lambda: dst.copy_(src)) / 1e3
+    del src, dst
+    print(f"device-to-device copy: {peak:.0f} GB/s (read + write)")
+    zdim, zc, temp = 20, 24, 0.6
+    alpha = torch.full((1,), 0.5, device=DEV)
+    for (n, hw, c) in [(512, 32, 64), (512, 16, 128), (512, 8, 256)]:
+        smp = ops.ConvLayer(1, 1, 1, 0, c, 2 * zdim, name="dec_sampler")
+        smp.w_tc = (torch.randn(2 * zdim, c, device=DEV, generator=g) * (0.7 / math.sqrt(c))).bfloat16().contiguous()
+        smp.bias = torch.randn(2 * zdim, device=DEV, generator=g) * 0.2
+        comb = ops.ConvLayer(1, 1, 1, 0, c, c, cin2=zc, name="dec_comb")
+        comb.w_tc = (torch.randn(c, c + zc, device=DEV, generator=g) / math.sqrt(c + zdim)).bfloat16().contiguous()
+        comb.bias = torch.randn(c, device=DEV, generator=g) * 0.2
+        x_elu = torch.nn.functional.elu(torch.randn(n, hw, hw, c, device=DEV, generator=g)).bfloat16()
+        xa = torch.randn(n, hw, hw, c, device=DEV, generator=g).bfloat16()
+        muq = torch.randn(n, hw, hw, zdim, device=DEV, generator=g)
+
+        def three():
+            pp = ops.conv2d_tc(x_elu, smp, want_bf16=False, want_f32=True)[1]
+            z = ops.latent_mix(muq, pp, None, 5, 3, 0, alpha, temp, zdim, zc, torch.bfloat16)
+            return ops.conv2d_tc(xa, comb, want_bf16=True, want_f32=True, x2=z)
+
+        t3 = timeit(three)
+        t1 = timeit(lambda: ops.latent_level(x_elu, xa, muq, None, smp, comb, 5, 3, 0, alpha, temp, zdim))
+        t1p = timeit(lambda: ops.latent_level(x_elu, xa, muq, None, smp, comb, 5, 3, 0, alpha, temp, zdim, want_pp=True))
+        m = n * hw * hw
+        by = m * (2 * c + 2 * c + 4 * zdim + 6 * c)
+        gbs = by / t1 / 1e3
+        print(f"level n={n} hw={hw} c={c}: three launches {t3:7.1f} us  fused {t1:7.1f} us ({by / 1e6:6.1f} MB, {gbs:5.0f} GB/s, "
+              f"{100 * gbs / peak:4.1f}% of copy)  fused + pp tape {t1p:7.1f} us  speed-up {t3 / t1:4.2f}x")
+
+
 if __name__ == "__main__":
     which = sys.argv[1:] or ["dwconv"]
     if "dwconv" in which:
@@ -189,3 +228,5 @@ if __name__ == "__main__":
         k1()
     if "hbm" in which:
         hbm()
+    if "level" in which:
+        level()
