@@ -227,7 +227,7 @@ def generator_synthesis(sd, latent, size: int):
 def mix_codes(sd_dec, codes, z_noise, alphas):
     """per-level latent interpolation, defenses/ours/models.py:117-127 / 329-342; z_noise (n, B, d) already scaled by its std"""
     styles = torch.stack([generator_style(sd_dec, n) for n in z_noise], dim=0)
-    a = torch.tensor(alphas, dtype=codes.dtype).view(-1, 1, 1)
+    a = torch.tensor(alphas, dtype=codes.dtype, device=codes.device).view(-1, 1, 1)
     return ((1 - a) * codes.permute(1, 0, 2) + a * styles).permute(1, 0, 2)
 
 

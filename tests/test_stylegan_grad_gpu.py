@@ -27,13 +27,21 @@ def rel_l2(a, b):
     return ((a - b).norm() / b.norm().clamp_min(1e-300)).item()
 
 
-def cosine(a, b):
-    a, b = a.detach().double().cpu().flatten(), b.detach().double().cpu().flatten()
-    return (a @ b / (a.norm() * b.norm())).item()
+def worst_code_rel_l2(a, b):
+    """largest rel-L2 of one code index of a (B, n_codes, 512) gradient: a wrong term in one layer moves its code's gradient by far more
+    than the whole gradient"""
+    a, b = a.detach().double().cpu(), b.detach().double().cpu()
+    return ((a - b).norm(dim=(0, 2)) / b.norm(dim=(0, 2)).clamp_min(1e-300)).max().item()
 
 
-def _d64(sd):
-    return {k: v.double() if v.is_floating_point() else v for k, v in sd.items()}
+def _d64(sd, device="cpu"):
+    return {k: v.to(device, torch.float64) if v.is_floating_point() else v.to(device) for k, v in sd.items()}
+
+
+def _bf16_ulp(t):
+    """spacing of bf16 numbers (8 significant bits) at |t|, elementwise, for float64 t"""
+    _, e = torch.frexp(t.abs())                                                # |t| = m 2^e, m in [0.5, 1)
+    return torch.ldexp(torch.ones_like(t), e - 8) * (t != 0)
 
 
 def _interleave(t4, n, h, w, c):
@@ -133,6 +141,58 @@ def test_phase_conv_dgrad_matches_modconv_upsample():
     assert rel_l2(g_x.permute(0, 3, 1, 2), ref) <= 1e-5
 
 
+@functools.lru_cache(maxsize=None)
+def _bf16_generator(size, cm):
+    eng = StyleGan2Engine(synth.make_stylegan2_state_dict(size, channel_multiplier=cm, seed=size + cm), size, DEV, "bf16",
+                          channel_multiplier=cm)
+    eng._build_adjoint()
+    return eng
+
+
+@pytest.mark.parametrize("out", ["bf16", "fp32"])
+@pytest.mark.parametrize("size,cm,j,up,n,h,w", [
+    (1024, 2, 7, False, 1, 1024, 1024),         # 32 -> 32 at 1024^2: the superpixel adjoint on the [n, H, W/2, 64] pair view
+    (512, 1, 6, False, 1, 512, 512),            # the same at 512^2 with channel_multiplier = 1
+    (1024, 2, 6, False, 1, 512, 512),           # plain 64 -> 64 dgrad at 512^2
+    (1024, 2, 5, False, 1, 256, 256),           # plain 128 -> 128 dgrad at 256^2
+    (1024, 2, 7, True, 1, 512, 512),            # up layer 512 -> 1024 (64 -> 32 ch): phase dgrad 128 -> 64 at 512^2
+    (1024, 2, 6, True, 1, 256, 256),            # up layer 256 -> 512 (128 -> 64 ch): phase dgrad 256 -> 128 at 256^2
+    (1024, 2, 6, False, 2, 136, 384),           # 64 -> 64 on two images of 17 x 12 windows of 8 x 32: window and image seams
+], ids=["sp1024", "sp512cm1", "c64at512", "c128at256", "up512to1024", "up256to512", "c64seams"])
+def test_adjoint_conv_bf16_shapes(size, cm, j, up, n, h, w, out):
+    """the conv adjoints the bf16 engine runs above f32_conv_out_res (tensor cores, wide-window mode of the persistent 3x3 kernel), built by
+    _build_adjoint and run through StyleGan2Engine._dgrad on a bf16 conv-output gradient, against autograd of F.conv2d in fp64 on the same
+    bf16-rounded operands (the forward layer's weights).  What is left is fp32 accumulation order and the output rounding, so the gate is
+    elementwise: one bf16 ulp of the reference (bf16 output) or 1e-5 max|ref| (fp32 output).  Max-abs, not rel-L2: one tap dropped at a
+    window seam moves a few border pixels only."""
+    eng = _bf16_generator(size, cm)
+    s = eng.blocks[j][0 if up else 1]
+    L = s.phase_convs if up else s.conv                                     # forward conv: [b, h, w, cin] -> [b, h, w, (4) cout]
+    f32 = out == "fp32"
+    g = torch.Generator(device=DEV).manual_seed(size + j + n)
+    g_y = torch.randn(n, h, w, L.cout, generator=g, device=DEV).to(torch.bfloat16)
+    sp = not up and s.conv_sp_d is not None and not f32
+    assert sp == (not up and s.cin == 32 and not f32)                       # the superpixel adjoint exists exactly for the 32-channel layers
+    D = s.conv_sp_d if sp else (s.phase_d if up else s.conv_d)
+    assert ops.conv2d_tc_supported(g_y.view(n, h, w // 2, 2 * L.cout) if sp else g_y, D)   # no silent fall-back to the SIMT kernel
+    got = eng._dgrad(s, g_y, f32)
+    assert got.dtype == (torch.float32 if f32 else torch.bfloat16) and got.shape == (n, h, w, L.cin)
+
+    wb = L.w_simt.view(3, 3, L.cin, L.cout).permute(3, 2, 0, 1).to(torch.bfloat16).double()
+    x = torch.zeros(n, L.cin, h, w, dtype=torch.float64, device=DEV, requires_grad=True)
+    ref, = torch.autograd.grad(F.conv2d(x, wb, padding=1), [x], g_y.double().permute(0, 3, 1, 2))
+    ref = ref.permute(0, 2, 3, 1)
+    err = (got.double() - ref).abs()
+    big = ref.abs().max().item()
+    if f32:
+        assert err.max().item() <= 1e-5 * big, err.max().item() / big
+    else:
+        # one ulp of the reference, plus 1e-6 max|ref| for the few sums that nearly cancel (there fp32 accumulation error can exceed the
+        # ulp); the floor is below one ulp of every element above 2.6e-4 max|ref|
+        bad = err > _bf16_ulp(ref) + 1e-6 * big
+        assert not bool(bad.any()), (int(bad.sum()), bad.nonzero()[:8].tolist(), (err / _bf16_ulp(ref)).max().item())
+
+
 # ------------------------------------------------------------------------------------------------ generator
 def _engine_branches(eng, tape):
     """the leaky-ReLU branch the engine's forward took in every styled layer (sign of its taped activation), whole batch, NCHW"""
@@ -171,7 +231,7 @@ def _oracle_branches(masks, cls=None):
         if x.dim() != 4:                                      # the mapping MLP (no gradient flows through it here)
             return orig(x, bias)
         t = x + bias.view(1, -1, 1, 1)
-        return torch.where(next(it), t, 0.2 * t) * math.sqrt(2.0)
+        return torch.where(next(it).to(t.device), t, 0.2 * t) * math.sqrt(2.0)
 
     class _Functional:
         """torch.nn.functional with the classifier's ReLUs and stem max-pool following the engine"""
@@ -185,10 +245,13 @@ def _oracle_branches(masks, cls=None):
         def relu(self, x):
             m = next(self.it)
             assert m.shape == x.shape, (m.shape, x.shape)
-            return torch.where(m, x, torch.zeros_like(x))
+            return torch.where(m.to(x.device), x, torch.zeros_like(x))
 
         def max_pool2d(self, x, k, s, p):
-            _, idx = F.max_pool2d(self.stem.to(x.dtype), k, s, p, return_indices=True)
+            # the element each window picks, from the engine's own stem output: the first maximum in scan order, which is also what
+            # maxpool3x3s2_bwd routes the gradient to, so ties (frequent in a bf16 stem) resolve alike
+            _, idx = F.max_pool2d(self.stem.contiguous(), k, s, p, return_indices=True)
+            idx = idx.to(x.device)
             return x.flatten(2).gather(2, idx.flatten(2)).view(idx.shape)
 
     stylegan_ref.fused_leaky_relu = fused_leaky_relu
@@ -203,40 +266,75 @@ def _oracle_branches(masks, cls=None):
 
 @functools.lru_cache(maxsize=None)
 def _synthesis_case(which):
-    """(state dict, size, latent, image gradient)"""
+    """(state dict, size, channel multiplier, latent, image gradient)"""
+    cm = 2
     if which == "golden32":
         gold = torch.load(GOLDEN, weights_only=True)
         size, sd = gold["size"], synth.make_stylegan2_state_dict(gold["size"], seed=gold["seed"])
-    else:
+    elif which == "synthetic256":
         size, sd = 256, synth.make_stylegan2_state_dict(256, seed=9)
+    elif which == "synthetic512cm1":
+        size, cm = 512, 1
+        sd = synth.make_stylegan2_state_dict(512, channel_multiplier=1, seed=10)
+    else:
+        size, sd = 1024, synth.make_stylegan2_state_dict(1024, seed=11)
     g = torch.Generator().manual_seed(size)
-    batch = 3 if size <= 32 else 2
+    batch = 2 if size == 256 else 3
     lat = torch.randn(batch, 2 * int(math.log2(size)) - 2, 512, generator=g)
-    return sd, size, lat, torch.randn(batch, 3, size, size, generator=g)
+    return sd, size, cm, lat, torch.randn(batch, 3, size, size, generator=g)
+
+
+def _mixed_slices(eng):
+    """blocks at >= 128^2 run on slices of 2 (a batch of 3: 2 + 1) while the lower resolutions run on the whole batch -- the engine's
+    recursive split at full size (_cap gives 16 images at 1024^2, 32 at 512^2) on a batch small enough for the fp64 oracle"""
+    eng.max_chunk = None
+    eng._cap = lambda j: 2 if (8 << j) >= 128 else 1 << 20
+
+
+# bf16 against the fp64 oracle on the engine's branches, measured on a B200: (rel-L2, worst rel-L2 of one code index); each gate is
+# about twice the measurement
+BF16_SYNTHESIS_GATES = {"golden32": (7e-3, 8e-3),             # measured 3.5e-3, 3.9e-3
+                        "synthetic256": (1e-2, 1.2e-2),         # 5.0e-3, 6.1e-3
+                        "synthetic512cm1": (1e-2, 1.7e-2),      # 4.9e-3, 8.6e-3
+                        "synthetic1024": (1.2e-2, 1.5e-2)}      # 6.1e-3, 7.4e-3
+MIXED = ("synthetic512cm1", "synthetic1024")
 
 
 @pytest.mark.parametrize("mode", ["fp32", "bf16"])
-@pytest.mark.parametrize("which", ["golden32", "synthetic256"])
+@pytest.mark.parametrize("which", ["golden32", "synthetic256", "synthetic512cm1", "synthetic1024"])
 def test_synthesis_backward(which, mode):
-    """the reverse sweep on batch slices of one sample (max_chunk = 1) against autograd through generator_synthesis in fp64 (fp32: on the
-    engine's leaky-ReLU branches; bf16: on the oracle's own)"""
-    sd, size, lat, g_img = _synthesis_case(which)
-    eng = StyleGan2Engine(sd, size, DEV, mode)
-    eng.max_chunk = 1
+    """the reverse sweep against autograd through generator_synthesis in fp64 on the engine's leaky-ReLU branches: on batch slices of one
+    sample (max_chunk = 1), and for 512^2 with channel_multiplier = 1 and for 1024^2 (32-channel superpixel layers) on mixed slices
+    (_mixed_slices: a ragged last slice, the low-resolution layers' dots written whole-batch, the high-resolution ones per slice)"""
+    sd, size, cm, lat, g_img = _synthesis_case(which)
+    eng = StyleGan2Engine(sd, size, DEV, mode, channel_multiplier=cm)
+    if which in MIXED:
+        _mixed_slices(eng)
+    else:
+        eng.max_chunk = 1
     tape = SynthesisTape()
     eng.synthesis(lat.to(DEV), tape=tape)
-    assert len(tape.slices) == lat.shape[0]
+    if which in MIXED:
+        assert tape.slices == [(0, 2), (2, 1)]
+        assert {k[1] for k in tape.acts if k[0] == id(eng.blocks[3][1])} == {0}          # 64^2: whole batch
+        assert {k[1] for k in tape.acts if k[0] == id(eng.blocks[4][0])} == {0, 2}       # 128^2: slices
+        assert (eng.blocks[-1][1].conv_sp is not None) == (mode == "bf16")                # 32 channels at the top: superpixel in bf16
+    else:
+        assert len(tape.slices) == lat.shape[0]
     g_nhwc = F.pad(g_img.permute(0, 2, 3, 1), (0, 1)).to(DEV)
     got = eng.synthesis_backward(tape, [g_nhwc[lo:lo + n].contiguous() for lo, n in tape.slices])
-    latd = lat.double().requires_grad_()
-    with _oracle_branches(_engine_branches(eng, tape)) if mode == "fp32" else contextlib.nullcontext():
-        img = stylegan_ref.generator_synthesis(_d64(sd), latd, size)
-    ref, = torch.autograd.grad((img * g_img.double()).sum(), [latd])
+    latd = lat.to(DEV, torch.float64).requires_grad_()
+    with _oracle_branches(_engine_branches(eng, tape)):
+        img = stylegan_ref.generator_synthesis(_d64(sd, DEV), latd, size)
+    ref, = torch.autograd.grad((img * g_img.to(img)).sum(), [latd])
     assert got.shape == ref.shape
+    err, worst = rel_l2(got, ref), worst_code_rel_l2(got, ref)
+    print(f"synthesis backward {which} {mode}: rel-L2 {err:.3e}, worst code {worst:.3e}")
     if mode == "fp32":
-        assert rel_l2(got, ref) <= 1e-4, rel_l2(got, ref)
+        assert err <= 1e-4, err
     else:
-        assert cosine(got, ref) >= 0.99, cosine(got, ref)
+        gate, gate_code = BF16_SYNTHESIS_GATES[which]
+        assert err <= gate and worst <= gate_code, (err, worst)
 
 
 # ------------------------------------------------------------------------------------------------ defenses
@@ -254,10 +352,10 @@ def _make_defense(kind, size, mode):
 
 def _ref_tail(kind, ck, clf_ck, codes, z, alphas, size):
     """the tail of e4e_defense_call / trans_defense_call from the codes: mix -> synthesis -> pool / crop / resize -> classifier, in the
-    codes' dtype"""
-    cast = _d64 if codes.dtype == torch.float64 else (lambda sd: sd)
+    codes' dtype, on the codes' device"""
+    cast = lambda sd: {k: v.to(codes.device, codes.dtype) if v.is_floating_point() else v.to(codes.device) for k, v in sd.items()}
     dec = cast(stylegan_ref._sub(ck["state_dict"], "decoder" if kind == "e4e" else "decoder.module"))
-    lat = stylegan_ref.mix_codes(dec, codes, z.to(codes.dtype) * (1.0 if kind == "e4e" else 0.8), alphas)
+    lat = stylegan_ref.mix_codes(dec, codes, z.to(codes) * (1.0 if kind == "e4e" else 0.8), alphas)
     img = F.adaptive_avg_pool2d(stylegan_ref.generator_synthesis(dec, lat, size), (256, 256))
     if kind != "e4e":
         img = img.clone()
@@ -268,8 +366,13 @@ def _ref_tail(kind, ck, clf_ck, codes, z, alphas, size):
     return stylegan_ref.resnet_forward(cast(clf_ck["state_dict"]), (pur - 0.5) / 0.5, 1 if kind == "e4e" else 32), pur
 
 
-def _check_from_codes(kind, size, batch, tol, ref_dtype=torch.float64):
-    dm, ck, clf_ck, alphas = _make_defense(kind, size, "fp32")
+def _check_from_codes(kind, size, batch, tol, mode="fp32", mixed_slices=False):
+    """from_codes forward and input gradient (preds_only both ways) against the fp64 oracle on the GPU, on the branches the engine's
+    generator and classifier took (from their tapes).  tol: rel-L2 gate of the gradient, or {preds_only: (rel-L2 gate, gate of the worst
+    code index)}"""
+    dm, ck, clf_ck, alphas = _make_defense(kind, size, mode)
+    if mixed_slices:
+        _mixed_slices(dm.autoencoder.decoder)
     n_codes = len(alphas)
     g = torch.Generator().manual_seed(size + batch)
     codes = torch.randn(batch, n_codes, 512, generator=g)
@@ -278,32 +381,46 @@ def _check_from_codes(kind, size, batch, tol, ref_dtype=torch.float64):
     dm.set_explicit_noise([torch.zeros(batch, 3, hw, hw), z])
     tape = CodesTape()
     dm._from_codes_cuda(codes.to(DEV), tape=tape)                             # the forward from_codes runs, for its branches
+    if mixed_slices:
+        assert tape.syn.slices == [(0, 2), (2, 1)]
     masks, cls = _engine_branches(dm.autoencoder.decoder, tape.syn), _classifier_branches(tape.cls)
     branches = lambda: _oracle_branches(masks, cls)
-    with branches():
-        logits_ref, pur_ref = _ref_tail(kind, ck, clf_ck, codes.to(ref_dtype).requires_grad_(), z, alphas, size)
-    g_l, g_p = torch.randn(logits_ref.shape, generator=g), torch.randn(pur_ref.shape, generator=g)
+    with branches(), torch.no_grad():
+        logits_ref, pur_ref = _ref_tail(kind, ck, clf_ck, codes.to(DEV, torch.float64), z, alphas, size)
+    g_l, g_p = torch.randn(logits_ref.shape, generator=g).to(DEV), torch.randn(pur_ref.shape, generator=g).to(DEV)
     for preds_only in (True, False):
         cd = codes.to(DEV).requires_grad_()
+        cr = codes.to(DEV, torch.float64).requires_grad_()
         if preds_only:
             logits = dm.from_codes(cd)
-            loss = (logits * g_l.to(DEV)).sum()
-            cr = codes.to(ref_dtype).requires_grad_()
+            loss = (logits * g_l).sum()
             with branches():
                 lr, _ = _ref_tail(kind, ck, clf_ck, cr, z, alphas, size)
-            ref, = torch.autograd.grad((lr * g_l.to(ref_dtype)).sum(), [cr])
+            ref, = torch.autograd.grad((lr * g_l.double()).sum(), [cr])
         else:
             logits, pur = dm.from_codes(cd, preds_only=False)
-            assert rel_l2(pur, pur_ref) <= 1e-4
-            loss = (logits * g_l.to(DEV)).sum() + (pur * g_p.to(DEV)).sum()
-            cr = codes.to(ref_dtype).requires_grad_()
+            if mode == "fp32":
+                assert rel_l2(pur, pur_ref) <= 1e-4
+            else:                                                           # the project's bf16 criterion on purified images in [0, 1]
+                assert (pur.double() - pur_ref).abs().max().item() <= 1e-2
+            loss = (logits * g_l).sum() + (pur * g_p).sum()
             with branches():
                 lr, pr = _ref_tail(kind, ck, clf_ck, cr, z, alphas, size)
-            ref, = torch.autograd.grad((lr * g_l.to(ref_dtype)).sum() + (pr * g_p.to(ref_dtype)).sum(), [cr])
-        # the fp32 forward (the same kernels as __call__) at the project's fp32 logits criterion (test_stylegan_paths_gpu.py)
-        assert (logits.detach().cpu().double() - logits_ref.detach().double()).abs().max() <= 1e-3 * logits_ref.detach().abs().max()
+            ref, = torch.autograd.grad((lr * g_l.double()).sum() + (pr * g_p.double()).sum(), [cr])
+        lerr = ((logits.detach().double() - logits_ref).abs().max() / logits_ref.abs().max()).item()
         got, = torch.autograd.grad(loss, [cd])
-        assert rel_l2(got, ref) <= tol, (kind, preds_only, rel_l2(got, ref))
+        err, worst = rel_l2(got, ref), worst_code_rel_l2(got, ref)
+        print(f"from_codes {kind} {size}^2 {mode} batch {batch} preds_only={preds_only}: logits max-abs / max {lerr:.3e}, "
+              f"gradient rel-L2 {err:.3e}, worst code {worst:.3e}")
+        if mode == "fp32":
+            # the fp32 forward (the same kernels as __call__) at the project's fp32 logits criterion (test_stylegan_paths_gpu.py)
+            assert lerr <= 1e-3, lerr
+            assert err <= tol, (kind, preds_only, err)
+        else:
+            # bf16 logits are reported only, as in test_classifier_grad_gpu.py: the random-init ResNets amplify bf16 rounding to about
+            # one logit unit (2e-2 of the cars logits, 0.8 of the small gender ones) even on the engine's branches
+            gate, gate_code = tol[preds_only]
+            assert err <= gate and worst <= gate_code, (kind, preds_only, err, worst)
     return dm
 
 
@@ -317,9 +434,22 @@ def test_from_codes_gradient(kind):
         dm(torch.rand(1, 3, hw, hw, device=DEV).requires_grad_())
 
 
-@pytest.mark.parametrize("kind,size", [("e4e", 1024), ("trans", 512)])
-def test_from_codes_gradient_full_size(kind, size):
-    _check_from_codes(kind, size, 1, 1e-4, ref_dtype=torch.float32)          # fp32 oracle: the fp64 one takes minutes at 1024^2
+# bf16 gradient against the fp64 oracle on the engine's branches, batch 3 on mixed slices, measured on a B200: {preds_only: (rel-L2,
+# worst rel-L2 of one code index)}; each gate is about twice the measurement
+BF16_FROM_CODES_GATES = {"e4e": {True: (3e-2, 4e-2),           # measured 1.55e-2, 1.94e-2
+                                False: (2.5e-2, 3e-2)},         # 1.23e-2, 1.46e-2
+                         "trans": {True: (3e-2, 3.3e-2),        # 1.44e-2, 1.64e-2
+                                   False: (3e-2, 3.3e-2)}}      # 1.41e-2, 1.64e-2
+
+
+@pytest.mark.parametrize("kind,size,mode", [("e4e", 1024, "fp32"), ("trans", 512, "fp32"), ("e4e", 1024, "bf16"), ("trans", 512, "bf16")],
+                         ids=["e4e-1024", "trans-512", "e4e-1024-bf16", "trans-512-bf16"])
+def test_from_codes_gradient_full_size(kind, size, mode):
+    """fp32: one sample; bf16 (the timed configuration): 3 samples, the generator's blocks at >= 128^2 on slices of 2 + 1"""
+    if mode == "fp32":
+        _check_from_codes(kind, size, 1, 1e-4)
+    else:
+        _check_from_codes(kind, size, 3, BF16_FROM_CODES_GATES[kind], mode="bf16", mixed_slices=True)
 
 
 @pytest.mark.parametrize("kind", ["e4e", "trans"])
