@@ -23,7 +23,7 @@ HEADER = os.path.join(ROOT_DIR, "include", "ga_b200.h")
 GA_F32, GA_BF16 = 0, 1
 PRE_NONE, PRE_ELU, PRE_SILU, PRE_AFFINE_SILU, PRE_AFFINE = 0, 1, 2, 3, 4
 ACT_NONE, ACT_SILU, ACT_ELU, ACT_RELU, ACT_LRELU_SQRT2, ACT_PRELU = 0, 1, 2, 3, 4, 5
-MUL_VALUE, MUL_RELU_MASK, MUL_ELU_FROM_Y = 0, 1, 2
+MUL_VALUE, MUL_RELU_MASK, MUL_ELU_FROM_Y, MUL_PRELU_FROM_Y = 0, 1, 2, 3
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-shared"]
@@ -128,6 +128,9 @@ _PROTOS = {
     "ga_sumpool2x2": (c_int, [T, T, T, c_void_p]),
     "ga_upsample_bilinear2x_bwd": (c_int, [T, T, c_void_p]),
     "ga_depth_to_space2": (c_int, [T, T, c_void_p]),
+    "ga_phase_interleave": (c_int, [T, T, T, c_int, c_void_p, T, c_void_p]),
+    "ga_subsample2x_bwd": (c_int, [T, T, c_void_p]),
+    "ga_codes_assemble_bwd": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_void_p]),
     "ga_maxpool3x3s2_bwd": (c_int, [T, T, c_int, T, c_void_p]),
     "ga_avgpool_bwd_relu": (c_int, [T, T, T, c_void_p]),
     "ga_maxpool2x2_bwd": (c_int, [T, T, c_int, T, c_void_p]),

@@ -86,6 +86,42 @@ class _CodesFn(torch.autograd.Function):
         return ctx.model._from_codes_backward(ctx.tape, g_preds, g_purified), None
 
 
+class ImagesTape:
+    """what `E4EStyleGanDefenseModel._to_codes_cuda` leaves behind: the pre-clamp image of the preprocessing, its blur flag, the encoder tape"""
+
+    def __init__(self):
+        from .irse_engine import EncoderTape
+        self.pre = None
+        self.blur = False
+        self.enc = EncoderTape()
+
+
+class _ImagesFn(torch.autograd.Function):
+    """`to_codes` of a StyleGAN defense as ONE node: images -> blur / noise / clamp / normalise -> encoder -> W+ codes.  Same contract as
+    _DefenseFn: the forward tapes, the backward runs the dgrad-only reverse sweep and leaves the tape intact (repeated backward works)."""
+
+    @staticmethod
+    def forward(ctx, batch, model):
+        tape = ImagesTape()
+        with torch.no_grad():
+            codes = model._to_codes_cuda(batch.detach(), tape=tape)
+        ctx.tape, ctx.model = tape, model
+        ctx.set_materialize_grads(False)
+        return codes
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, g_codes):
+        if g_codes is None:
+            return None, None
+        return ctx.model._to_codes_backward(ctx.tape, g_codes), None
+
+
+def images_apply(model, batch: torch.Tensor):
+    """differentiable `_StyleGanDefenseBase.to_codes` body -> codes"""
+    return _ImagesFn.apply(batch, model)
+
+
 def codes_apply(model, codes: torch.Tensor):
     """differentiable `_StyleGanDefenseBase.from_codes` body -> (preds, purified)"""
     return _CodesFn.apply(codes, model)

@@ -89,7 +89,7 @@ __global__ void __launch_bounds__(256) add_f32x4_kernel(const float4* __restrict
 }
 
 // ---------------------------------------------------------------------------- SE + residual backward
-// forward: out = skip + s * gate[n,c] * r ;  gate = sigmoid(W2 relu(W1 mean(r) + b1) + b2)
+// forward: out = skip + s * gate[n,c] * r ;  gate = sigmoid(W2 relu(W1 mean(r) + b1) + b2)   (b1 / b2 may be null: no bias)
 // stage 1: dots[n][blk][c] = sum over the block's pixel slice of g_out * r
 __global__ void __launch_bounds__(256) se_bwd_reduce_kernel(const void* __restrict__ g, int g_dtype, const void* __restrict__ r,
                                                             int r_dtype, int HW, int C, int pix_per_block,
@@ -198,11 +198,11 @@ __global__ void __launch_bounds__(256) se_bwd_apply_kernel(SeBwdParams p) {
     float a = 0.f;
     for (int c = lane; c < p.C; c += 32) a = fmaf(p.w1[(int64_t)j * p.C + c], s_mean[c], a);
     a = warp_sum(a);
-    if (lane == 0) s_hid[j] = a + p.b1[j];          // pre-ReLU
+    if (lane == 0) s_hid[j] = a + (p.b1 != nullptr ? p.b1[j] : 0.f);          // pre-ReLU
   }
   __syncthreads();
   for (int c = tid; c < p.C; c += 256) {
-    float a = p.b2[c];
+    float a = p.b2 != nullptr ? p.b2[c] : 0.f;
     for (int j = 0; j < p.hidden; ++j) a = fmaf(p.w2[(int64_t)c * p.hidden + j], fmaxf(s_hid[j], 0.f), a);
     const float gt = sigmoidf_(a);
     s_gate[c] = gt;
@@ -323,6 +323,56 @@ __global__ void __launch_bounds__(256) depth_to_space2_kernel(const float4* __re
   const int64_t n = t / (2 * h);
   const int ph = (Y & 1) * 2 + (X & 1);
   out[idx] = __ldg(in + (((n * h + (Y >> 1)) * w + (X >> 1)) * 4 + ph) * c4 + c);
+}
+
+// depth_to_space2 with the rest of the dgrad epilogue: out = (d2s(in) + add) * f(mul), fp32 in, fp32 / bf16 out.  One pass over the four
+// phases of a stride-2 conv's input gradient instead of d2s, add and mask as three; same arithmetic, in the same order, as those three.
+template <typename TOut>
+__global__ void __launch_bounds__(256) phase_interleave_kernel(const float4* __restrict__ in, const void* add, int add_dtype, const void* mul,
+                                                               int mul_dtype, int mul_mode, const float* __restrict__ slope, TOut* __restrict__ out,
+                                                               int64_t total4, int h, int w, int c4) {
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;      // over the OUTPUT, 4-channel vectors
+  if (idx >= total4) return;
+  const int c = (int)(idx % c4);
+  int64_t t = idx / c4;
+  const int X = (int)(t % (2 * w)); t /= 2 * w;
+  const int Y = (int)(t % (2 * h));
+  const int64_t n = t / (2 * h);
+  const int ph = (Y & 1) * 2 + (X & 1);
+  const float4 v4 = __ldg(in + (((n * h + (Y >> 1)) * w + (X >> 1)) * 4 + ph) * c4 + c);
+  float v[4] = {v4.x, v4.y, v4.z, v4.w};
+  const int64_t i = idx * 4;
+  if (add != nullptr) {
+    float a[4];
+    if (add_dtype == GA_F32) ld4<float>(reinterpret_cast<const float*>(add) + i, a); else ld4<__nv_bfloat16>(reinterpret_cast<const __nv_bfloat16*>(add) + i, a);
+#pragma unroll
+    for (int j = 0; j < 4; ++j) v[j] += a[j];
+  }
+  if (mul != nullptr) {
+    float m[4];
+    if (mul_dtype == GA_F32) ld4<float>(reinterpret_cast<const float*>(mul) + i, m); else ld4<__nv_bfloat16>(reinterpret_cast<const __nv_bfloat16*>(mul) + i, m);
+#pragma unroll
+    for (int j = 0; j < 4; ++j) v[j] *= mul_factor(m[j], mul_mode, slope != nullptr ? __ldg(slope + 4 * c + j) : 0.f);
+  }
+  st4<TOut>(out + i, v);
+}
+
+// adjoint of the stride-2 sub-sample (MaxPool2d(1, 2)): every output pixel is written, the odd ones with zeros
+__global__ void __launch_bounds__(256) subsample2x_bwd_kernel(const void* g, int g_dtype, void* out, int out_dtype, int64_t total4, int H, int W,
+                                                              int c4, int Hg, int Wg) {
+  const int64_t idx = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= total4) return;
+  const int c = (int)(idx % c4);
+  int64_t t = idx / c4;
+  const int x = (int)(t % W); t /= W;
+  const int y = (int)(t % H);
+  const int64_t n = t / H;
+  float v[4] = {0.f, 0.f, 0.f, 0.f};
+  if (((x | y) & 1) == 0) {
+    const int64_t gi = ((n * Hg + (y >> 1)) * Wg + (x >> 1)) * (4 * c4) + 4 * c;
+    if (g_dtype == GA_F32) ld4<float>(reinterpret_cast<const float*>(g) + gi, v); else ld4<__nv_bfloat16>(reinterpret_cast<const __nv_bfloat16*>(g) + gi, v);
+  }
+  if (out_dtype == GA_F32) st4<float>(reinterpret_cast<float*>(out) + idx * 4, v); else st4<__nv_bfloat16>(reinterpret_cast<__nv_bfloat16*>(out) + idx * 4, v);
 }
 
 // transpose of the align_corners=True bilinear x2 up-sampling, as a deterministic gather
@@ -732,7 +782,7 @@ extern "C" int ga_add(const ga_tensor* a, const ga_tensor* b, const ga_tensor* o
 extern "C" int ga_se_residual_bwd(const ga_tensor* g_out, const ga_tensor* r, const float* sums, float* dots_ws, const float* w1,
                                   const float* b1, const float* w2, const float* b2, int hidden, float res_scale,
                                   const ga_tensor* g_r, void* stream) {
-  GA_CHECK(g_out && r && sums && dots_ws && w1 && b1 && w2 && b2 && g_r, "ga_se_residual_bwd: null argument");
+  GA_CHECK(g_out && r && sums && dots_ws && w1 && w2 && g_r, "ga_se_residual_bwd: null argument");
   GA_CHECK(same_shape(g_out, r) && same_shape(g_out, g_r), "ga_se_residual_bwd: shape mismatch");
   if (numel(r) == 0) return 0;
   const int HW = r->h * r->w, C = r->c;
@@ -784,6 +834,42 @@ extern "C" int ga_depth_to_space2(const ga_tensor* in, const ga_tensor* out, voi
   if (total4 == 0) return 0;
   depth_to_space2_kernel<<<cdiv(total4, 256), 256, 0, (cudaStream_t)stream>>>((const float4*)in->data, (float4*)out->data, total4, in->h,
                                                                               in->w, out->c / 4);
+  GA_LAUNCH_OK();
+  return 0;
+}
+
+extern "C" int ga_phase_interleave(const ga_tensor* in, const ga_tensor* add, const ga_tensor* mul, int mul_mode, const float* slope,
+                                   const ga_tensor* out, void* stream) {
+  GA_CHECK(in && out && in->dtype == GA_F32, "ga_phase_interleave: fp32 input expected");
+  GA_CHECK(out->n == in->n && out->h == 2 * in->h && out->w == 2 * in->w && in->c == 4 * out->c && out->c % 4 == 0,
+           "ga_phase_interleave: shape mismatch (in [n,h,w,4c] -> out [n,2h,2w,c], c % 4 == 0)");
+  GA_CHECK(!add || same_shape(add, out), "ga_phase_interleave: add shape mismatch");
+  GA_CHECK(!mul || same_shape(mul, out), "ga_phase_interleave: mul shape mismatch");
+  GA_CHECK(!mul || mul_mode != GA_MUL_PRELU_FROM_Y || slope, "ga_phase_interleave: PReLU mask needs slope");
+  auto aligned = [](const ga_tensor* t) { return !t || (((uintptr_t)t->data) & (t->dtype == GA_F32 ? 15 : 7)) == 0; };
+  GA_CHECK(aligned(in) && aligned(out) && aligned(add) && aligned(mul), "ga_phase_interleave: tensors must be 4-channel-vector aligned");
+  const int64_t total4 = numel(out) / 4;
+  if (total4 == 0) return 0;
+  const int ad = add ? add->dtype : GA_F32, md = mul ? mul->dtype : GA_F32;
+  if (out->dtype == GA_F32)
+    phase_interleave_kernel<float><<<cdiv(total4, 256), 256, 0, (cudaStream_t)stream>>>(
+        (const float4*)in->data, add ? add->data : nullptr, ad, mul ? mul->data : nullptr, md, mul_mode, slope, (float*)out->data, total4, in->h,
+        in->w, out->c / 4);
+  else
+    phase_interleave_kernel<__nv_bfloat16><<<cdiv(total4, 256), 256, 0, (cudaStream_t)stream>>>(
+        (const float4*)in->data, add ? add->data : nullptr, ad, mul ? mul->data : nullptr, md, mul_mode, slope, (__nv_bfloat16*)out->data, total4,
+        in->h, in->w, out->c / 4);
+  GA_LAUNCH_OK();
+  return 0;
+}
+
+extern "C" int ga_subsample2x_bwd(const ga_tensor* g, const ga_tensor* out, void* stream) {
+  GA_CHECK(g && out && g->n == out->n && g->c == out->c && g->h == (out->h + 1) / 2 && g->w == (out->w + 1) / 2 && out->c % 4 == 0,
+           "ga_subsample2x_bwd: shape mismatch (g [n,ceil(h/2),ceil(w/2),c] -> out [n,h,w,c], c % 4 == 0)");
+  const int64_t total4 = numel(out) / 4;
+  if (total4 == 0) return 0;
+  subsample2x_bwd_kernel<<<cdiv(total4, 256), 256, 0, (cudaStream_t)stream>>>(g->data, g->dtype, out->data, out->dtype, total4, out->h, out->w,
+                                                                              out->c / 4, g->h, g->w);
   GA_LAUNCH_OK();
   return 0;
 }

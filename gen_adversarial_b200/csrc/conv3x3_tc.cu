@@ -97,7 +97,7 @@ __global__ void __launch_bounds__(C3_THREADS, 1) conv3x3_tc_kernel(const __grid_
     const int et = threadIdx.x - 64;
     for (int i = et; i < n_blocks * BLOCK_N; i += 128) {
       s_bias[i] = (p.bias != nullptr && i < p.cout) ? p.bias[i] : 0.f;
-      if (GENERAL_ACT) s_slope[i] = (p.act_slope != nullptr && i < p.cout) ? p.act_slope[i] : 0.f;
+      if (GENERAL_ACT || (EPI == 3 && p.mul_mode == GA_MUL_PRELU_FROM_Y)) s_slope[i] = (p.act_slope != nullptr && i < p.cout) ? p.act_slope[i] : 0.f;
     }
   }
   tc_fence_before();
@@ -238,7 +238,7 @@ __global__ void __launch_bounds__(C3_THREADS, 1) conv3x3_tc_kernel(const __grid_
                                     pixw0 + s * pixw_s, s_stage, s_bias + n_blk * BLOCK_N, q, lane, s_csum + s * (4 * BLOCK_N));
         else if (EPI == 3)
           tc_epilogue_lean_am<BLOCK_N>(p, &tmOutB, &tmOutF, tmem_base + buf * (2 * BLOCK_N) + s * BLOCK_N, n_blk,
-                                       pixw0 + s * pixw_s, s_stage, s_bias + n_blk * BLOCK_N, q, lane);
+                                       pixw0 + s * pixw_s, s_stage, s_bias + n_blk * BLOCK_N, s_slope + n_blk * BLOCK_N, q, lane);
         else
           tc_epilogue_tile<BLOCK_N, GENERAL_ACT, true>(p, &tmOutB, &tmOutF, &tmOutD, tmem_base + buf * (2 * BLOCK_N) + s * BLOCK_N, n_blk,
                                                        pixw0 + s * pixw_s, 128, s_stage, s_bias + n_blk * BLOCK_N,
@@ -376,8 +376,9 @@ int conv3x3_halo_launch(const ga_tensor* in, const void* weight, int ktot, const
   C3Plan pl;
   p.cin = cin; p.cout = cout; p.tma_store = 1; p.partial = 0;
   const bool general = p.act_after_add != 0 || p.post_act == GA_ACT_PRELU;
+  const bool prelu_mask = p.mul != nullptr && p.mul_mode == GA_MUL_PRELU_FROM_Y;     // needs the slopes: lean add/mul epilogue or the general one
   const int epi = general ? 2 : ((lean_enabled() && tc_epilogue_is_lean(p) && !(p.dact && out_f32 && !out_bf16)) ? 0 :
-                                 ((lean_enabled() && tc_epilogue_is_lean_am(p)) ? 3 : 1));
+                                 ((lean_enabled() && tc_epilogue_is_lean_am(p)) ? 3 : (prelu_mask ? 2 : 1)));
   if (!c3_plan(in->n, H, W, cin, cout, out_bf16 != nullptr, out_f32 != nullptr, p.dact != nullptr, epi == 0, &pl)) return -1;
   if (out_bf16 && (((uintptr_t)out_bf16->data) & 15)) return -1;
   if (out_f32 && (((uintptr_t)out_f32->data) & 15)) return -1;
@@ -445,7 +446,7 @@ int conv1x1_persistent_launch(const ga_tensor* in, const void* weight, int ktot,
   if (out_f32 && (((uintptr_t)out_f32->data) & 15)) return -1;
   if (p.dact && (((uintptr_t)p.dact) & 15)) return -1;
   p.cin = cin; p.cout = cout; p.tma_store = 1; p.partial = 0; p.M = M; p.H = in->h; p.W = in->w;
-  if (p.act_after_add != 0 || p.post_act == GA_ACT_PRELU) return -1;
+  if (p.act_after_add != 0 || p.post_act == GA_ACT_PRELU || (p.mul != nullptr && p.mul_mode == GA_MUL_PRELU_FROM_Y)) return -1;
   int epi;
   if (tc_epilogue_is_lean(p) && !(p.dact && out_f32 && !out_bf16)) epi = 0;
   // add/mul epilogues stream one more tensor per output row: with one CTA per SM and four epilogue warps too few of those loads are in flight

@@ -201,7 +201,7 @@ __global__ void __launch_bounds__(NT) conv_igemm_simt_kernel(ConvParams p) {
         if (p.mul != nullptr) {
           const float mv = (p.mul_dtype == GA_F32) ? reinterpret_cast<const float*>(p.mul)[off + j]
                                                    : __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(p.mul)[off + j]);
-          r *= mul_factor(mv, p.mul_mode);
+          r *= mul_factor(mv, p.mul_mode, slope);
         }
         stf<TOut>(out + off + j, r);
       }
@@ -371,6 +371,7 @@ extern "C" int ga_conv2d_simt(const ga_tensor* in, const ga_conv_desc* d, const 
   p.dact = d->dact_out; p.dact_dtype = d->dact_dtype;
   p.act_slope = d->act_slope; p.act_after_add = d->act_after_add;
   GA_CHECK(d->post_act != GA_ACT_PRELU || d->act_slope != nullptr, "ga_conv2d_simt: PReLU needs act_slope");
+  GA_CHECK(d->mul == nullptr || d->mul_mode != GA_MUL_PRELU_FROM_Y || d->act_slope != nullptr, "ga_conv2d_simt: PReLU mask needs act_slope");
   p.out = out->data;
   p.N = in->n; p.H = in->h; p.W = in->w; p.Cin = in->c; p.Ho = out->h; p.Wo = out->w; p.Cout = out->c;
   p.KH = d->kh; p.KW = d->kw; p.stride = d->stride; p.pad = d->pad; p.up = d->up;

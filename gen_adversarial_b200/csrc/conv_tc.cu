@@ -261,7 +261,8 @@ static int launch_tc_(const CUtensorMap& a, const CUtensorMap& a2, const CUtenso
 template <int BLOCK_N, int STAGES>
 static int launch_tc(const CUtensorMap& a, const CUtensorMap& a2, const CUtensorMap& b, const CUtensorMap& ob, const CUtensorMap& of,
                      const CUtensorMap& od, const TcParams& p, dim3 grid, cudaStream_t s) {
-  if (p.act_after_add != 0 || p.post_act == GA_ACT_PRELU) return launch_tc_<BLOCK_N, STAGES, true>(a, a2, b, ob, of, od, p, grid, s);
+  if (p.act_after_add != 0 || p.post_act == GA_ACT_PRELU || (p.mul != nullptr && p.mul_mode == GA_MUL_PRELU_FROM_Y))
+    return launch_tc_<BLOCK_N, STAGES, true>(a, a2, b, ob, of, od, p, grid, s);
   return launch_tc_<BLOCK_N, STAGES, false>(a, a2, b, ob, of, od, p, grid, s);
 }
 
@@ -341,6 +342,7 @@ extern "C" int ga_conv2d_tc(const ga_tensor* in, const ga_tensor* in2, const ga_
   p.round_tf32 = (out_f32 && round_tf32_enabled()) ? 1 : 0;
   p.csum = d->csum_out;
   GA_CHECK(d->post_act != GA_ACT_PRELU || d->act_slope != nullptr, "ga_conv2d_tc: PReLU needs act_slope");
+  GA_CHECK(d->mul == nullptr || d->mul_mode != GA_MUL_PRELU_FROM_Y || d->act_slope != nullptr, "ga_conv2d_tc: PReLU mask needs act_slope");
   // 3x3 stride-1 convolutions on 64-channel blocks: persistent halo-reuse kernel (conv3x3_tc.cu); -1 = shape not covered there
   if (d->kh == 3 && d->kw == 3 && d->stride == 1 && d->pad == 1 && !in2 && !tf32 && !k32) {
     const int rc = conv3x3_halo_launch(in, d->weight, ktot, out_bf16, out_f32, p, (cudaStream_t)stream);

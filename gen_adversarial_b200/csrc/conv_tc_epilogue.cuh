@@ -44,7 +44,8 @@ bool conv3x3_halo_csum_ok(const ga_tensor* in, int cout, const TcParams& p, bool
 
 // tmem_acc: TMEM address (lane 0) of column 0 of the accumulator; pix0: global index of the tile's first output pixel; row_limit: rows of
 // the tile that exist (128, or fewer for the partial last tile row of an image); stage: 1024-aligned staging memory (TMA-store mode);
-// s_bias / s_slope: BLOCK_N floats each in shared memory (bias and PReLU slopes of this N block).
+// s_bias / s_slope: BLOCK_N floats each in shared memory (bias and PReLU slopes of this N block; GENERAL_ACT only).  The slopes serve
+// post_act = GA_ACT_PRELU and mul_mode = GA_MUL_PRELU_FROM_Y alike: the host runs both on GENERAL_ACT instantiations.
 // DEFER_STORE_WAIT: return without waiting for the bulk stores to have read the staging tile (the caller waits before re-using it).
 // LD_COLS: accumulator columns fetched per tcgen05.ld round trip.  A round trip costs ~1k cycles while the tensor pipe is busy (measured: the
 // persistent 3x3 kernel spent 1000 clk per 16-column chunk); a kernel with few resident warps must put many columns in flight per wait.
@@ -109,8 +110,12 @@ __device__ __forceinline__ void tc_epilogue_tile(const TcParams& p, const CUtens
     } else if (!GENERAL_ACT) {
       apply_act_fast_n<16>(v, p.post_act);
     } else if (!p.act_after_add) {
+      if (p.post_act == GA_ACT_PRELU) {
 #pragma unroll
-      for (int j = 0; j < 16; ++j) v[j] = v[j] > 0.f ? v[j] : s_slope[c0 + j] * v[j];
+        for (int j = 0; j < 16; ++j) v[j] = v[j] > 0.f ? v[j] : s_slope[c0 + j] * v[j];
+      } else {
+        apply_act_fast_n<16>(v, p.post_act);
+      }
     }
     if (p.add != nullptr && row_ok) {
       if (full) {
@@ -167,14 +172,14 @@ __device__ __forceinline__ void tc_epilogue_tile(const TcParams& p, const CUtens
         }
       }
 #pragma unroll
-      for (int j = 0; j < 16; ++j) v[j] *= mul_factor(mv[j], p.mul_mode);
+      for (int j = 0; j < 16; ++j) v[j] *= mul_factor(mv[j], p.mul_mode, GENERAL_ACT ? s_slope[c0 + j] : 0.f);
     } else if (p.mul != nullptr && row_ok) {
 #pragma unroll
       for (int j = 0; j < 16; ++j) {
         if (nb + j < p.cout) {
           const float mv = (p.mul_dtype == GA_F32) ? __ldg(reinterpret_cast<const float*>(p.mul) + off + j)
                                                    : __bfloat162float(reinterpret_cast<const __nv_bfloat16*>(p.mul)[off + j]);
-          v[j] *= mul_factor(mv, p.mul_mode);
+          v[j] *= mul_factor(mv, p.mul_mode, GENERAL_ACT ? s_slope[c0 + j] : 0.f);
         }
       }
     }
@@ -432,7 +437,7 @@ __device__ __forceinline__ void tc_epilogue_lean(const TcParams& p, const CUtens
 }
 
 // Lean epilogue with the backward-pass extras: out = (act(acc + bias) + add) * f(mul), add / mul tensors of the output's shape in fp32 or
-// bf16.  Each thread owns one output row: its add / mul values of the whole 64-column group are fetched with 16-byte loads BEFORE the
+// bf16; f(mul) is one of the ga_mul_mode factors (PReLU: s_slope holds this N block's slopes).  Each thread owns one output row: its add / mul values of the whole 64-column group are fetched with 16-byte loads BEFORE the
 // tcgen05.wait, so the global-load latency overlaps the TMEM round trip (the generic epilogue loads them per 16-column chunk, after the math).
 __host__ __device__ __forceinline__ bool tc_epilogue_is_lean_am(const TcParams& p) {
   return (p.add != nullptr || p.mul != nullptr) && p.act_after_add == 0 && p.tma_store != 0 && p.round_tf32 == 0 && p.dact == nullptr &&
@@ -441,7 +446,8 @@ __host__ __device__ __forceinline__ bool tc_epilogue_is_lean_am(const TcParams& 
 
 template <int BLOCK_N>
 __device__ __forceinline__ void tc_epilogue_lean_am(const TcParams& p, const CUtensorMap* tmOutB, const CUtensorMap* tmOutF, uint32_t tmem_acc,
-                                                    int n_blk, int64_t pix0, uint8_t* stage, const float* s_bias, int q, int lane) {
+                                                    int n_blk, int64_t pix0, uint8_t* stage, const float* s_bias, const float* s_slope,
+                                                    int q, int lane) {
   constexpr int LD = BLOCK_N < 64 ? BLOCK_N : 64;
   const int row = q * 32 + lane;
   const int64_t pix = pix0 + row;
@@ -536,6 +542,9 @@ __device__ __forceinline__ void tc_epilogue_lean_am(const TcParams& p, const CUt
         } else if (p.mul_mode == GA_MUL_ELU_FROM_Y) {
 #pragma unroll
           for (int j = 0; j < 16; ++j) v[j] *= (mv[j] > 0.0f ? 1.0f : mv[j] + 1.0f);
+        } else if (p.mul_mode == GA_MUL_PRELU_FROM_Y) {
+#pragma unroll
+          for (int j = 0; j < 16; ++j) v[j] *= (mv[j] > 0.0f ? 1.0f : s_slope[c0 + j]);
         } else {
 #pragma unroll
           for (int j = 0; j < 16; ++j) v[j] *= mv[j];

@@ -157,6 +157,23 @@ __global__ void codes_assemble_kernel(const float* __restrict__ heads, int heads
   out[i] = v;
 }
 
+// adjoint of codes_assemble (heads_lb, use_w0): g_heads[l][b][d] = g_codes[b][l][d] (l > 0), g_heads[0][b][d] = sum_l g_codes[b][l][d]
+// in increasing l (one thread per (b, d): fixed order, no atomics, independent of the batch size)
+__global__ void codes_assemble_bwd_kernel(const float* __restrict__ g, int B, int L, int D, float* __restrict__ out) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= (int64_t)B * D) return;
+  const int d = (int)(i % D);
+  const int64_t b = i / D;
+  const float* gb = g + b * L * D + d;
+  float s = 0.f;
+  for (int l = 0; l < L; ++l) {
+    const float v = gb[(int64_t)l * D];
+    s += v;
+    if (l > 0) out[((int64_t)l * B + b) * D + d] = v;
+  }
+  out[b * D + d] = s;
+}
+
 // ---------------------------------------------------------------------------- bilinear resize (align_corners=False, no antialias) + row crop
 // out[n, y, x, c] = bilinear(in[n], (y + crop_y0 + 0.5) * H/Hfull - 0.5, (x + 0.5) * W/Wo - 0.5)   (F.interpolate semantics)
 __global__ void resize_bilinear_kernel(const void* in, int in_dtype, int N, int H, int W, int C, int Hfull, int crop_y0, int Ho, int Wo,
@@ -291,6 +308,15 @@ extern "C" int ga_codes_assemble(const float* heads, int heads_lb, int use_w0, c
   const int64_t total = (int64_t)b * l * d;
   if (total == 0) return 0;
   codes_assemble_kernel<<<cdiv(total, 256), 256, 0, (cudaStream_t)stream>>>(heads, heads_lb, use_w0, latent_avg, b, l, d, out);
+  GA_LAUNCH_OK();
+  return 0;
+}
+
+extern "C" int ga_codes_assemble_bwd(const float* g_codes, int b, int l, int d, float* g_heads, void* stream) {
+  GA_CHECK(g_codes && g_heads && b >= 0 && l >= 1 && d >= 1, "ga_codes_assemble_bwd: bad arguments");
+  const int64_t total = (int64_t)b * d;
+  if (total == 0) return 0;
+  codes_assemble_bwd_kernel<<<cdiv(total, 256), 256, 0, (cudaStream_t)stream>>>(g_codes, b, l, d, g_heads);
   GA_LAUNCH_OK();
   return 0;
 }

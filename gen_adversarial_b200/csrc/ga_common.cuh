@@ -220,10 +220,12 @@ __device__ __forceinline__ float2 ffma2(float2 a, float2 b, float2 c) {
   return *reinterpret_cast<float2*>(&d);
 }
 
-__device__ __forceinline__ float mul_factor(float m, int mode) {
+// slope: PReLU slope of m's channel (GA_MUL_PRELU_FROM_Y only)
+__device__ __forceinline__ float mul_factor(float m, int mode, float slope) {
   switch (mode) {
     case GA_MUL_RELU_MASK: return m > 0.0f ? 1.0f : 0.0f;
     case GA_MUL_ELU_FROM_Y: return m > 0.0f ? 1.0f : m + 1.0f;
+    case GA_MUL_PRELU_FROM_Y: return m > 0.0f ? 1.0f : slope;
     default: return m;
   }
 }

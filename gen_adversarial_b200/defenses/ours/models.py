@@ -170,12 +170,16 @@ class _StyleGanDefenseBase(MLVGMDefenseModel):
             raise ValueError(f"{len(self.interpolation_alphas)} interpolation alphas for {n} codes")
         return self.autoencoder.decoder.mix_codes(codes, self._style_noise(n, b, d), self._alphas_device())
 
-    def _preprocessed(self, batch, normalize=True):
+    def _preprocessed(self, batch, normalize=True, tape=None):
+        """tape: an `autograd.ImagesTape` receiving the pre-clamp image and the blur flag for the backward"""
         noise0 = self._explicit_noise[0] if self._explicit_noise is not None else None
         self._seed_now = self._next_seed()
         # fp32 image into the encoder stem (a 3-channel SIMT conv either way): a bf16 input would perturb the image by up to 2e-3
-        x, _ = ops.preprocess(batch.detach().to(torch.float32), noise0, float(self.eps), bool(self.blur_input), torch.float32,
-                              seed=self._seed_now, sample0=self.sample_offset, normalize=normalize, taps_cache=self._taps_cache)
+        x, pre = ops.preprocess(batch.detach().to(torch.float32), noise0, float(self.eps), bool(self.blur_input), torch.float32,
+                                seed=self._seed_now, sample0=self.sample_offset, normalize=normalize, save_pre=tape is not None,
+                                taps_cache=self._taps_cache)
+        if tape is not None:
+            tape.pre, tape.blur = pre, bool(self.blur_input)
         return x
 
     def _decode(self, codes, cls_dtype, want_purified=True, denorm=(0.5, 0.5), tape=None):
@@ -205,6 +209,18 @@ class _StyleGanDefenseBase(MLVGMDefenseModel):
         codes = self._mix(self._encode(x))
         purified, cls_in = self._decode(codes, self.classifier.classifier.adt)
         return self.classifier.classifier.forward(cls_in), purified
+
+    def to_codes(self, batch: torch.Tensor) -> torch.Tensor:
+        """The head of `__call__`: images (B, 3, H, W) in [0, 1] -> blur / L2 noise / clamp / normalise -> encoder -> W+ codes
+        (B, n_codes, 512) fp32, before the style-noise mix (what `from_codes` takes).  The preprocessing draws one seed, with the same
+        `sample_offset`, explicit-noise and `noise_seed` rules as a call; `from_codes` draws another for the style noise.  So with explicit
+        noise, or with `noise_seed` set, `from_codes(to_codes(x))` gives the logits of `__call__(x)`.
+        Differentiable w.r.t. `batch` (input gradient only; repeated backward through one forward works) for the E4E defense; the
+        Style-Transformer encoder has no backward yet and refuses when a gradient is needed."""
+        if batch.requires_grad and torch.is_grad_enabled():
+            from ...autograd import images_apply
+            return images_apply(self, batch)
+        return self._encode(self._preprocessed(batch))
 
     def from_codes(self, codes: torch.Tensor, preds_only: bool = True):
         """The tail of `__call__` from the encoder's W+ codes (B, n_codes, 512) fp32: mix with the style noise (same seed / explicit-noise /
@@ -271,6 +287,17 @@ class E4EStyleGanDefenseModel(_StyleGanDefenseBase, torch.nn.Module):
     def _encode(self, x_nhwc):
         return self.autoencoder.encoder.encode(x_nhwc)                                    # psp.py:88-101
 
+    def _to_codes_cuda(self, batch: torch.Tensor, tape):
+        """-> codes; tape: an `autograd.ImagesTape` to fill for `_to_codes_backward`"""
+        self.autoencoder.encoder.build_dgrad()            # before any launch: refuses a checkpoint whose PReLU masks cannot be recovered
+        x = self._preprocessed(batch, tape=tape)
+        return self.autoencoder.encoder.encode(x, tape=tape.enc)
+
+    def _to_codes_backward(self, tape, g_codes: torch.Tensor) -> torch.Tensor:
+        """d loss / d codes (B, n_codes, 512) -> d loss / d images (B, 3, H, W) fp32"""
+        g_x = self.autoencoder.encoder.encode_backward(tape.enc, g_codes.contiguous().to(torch.float32))
+        return ops.preprocess_bwd(g_x, tape.pre, tape.blur, normalize=True, taps_cache=self._taps_cache)
+
     def _pool_out(self, img, cls_dtype, want_purified, denorm):
         k = img.shape[1] // 256                                                           # face_pool -> 256 x 256, psp.py:26,114
         return ops.image_pool_out(img, k, 1, 0, denorm, cls_dtype, want_purified)
@@ -303,6 +330,10 @@ class TransStyleGanDefenseModel(_StyleGanDefenseBase, torch.nn.Module):
         enc = TransEncoderEngine(_sub_state_dict(ckpt["state_dict"], "encoder.module"), lat, device, self._mode)
         dec = StyleGan2Engine(_sub_state_dict(ckpt["state_dict"], "decoder.module"), size, device, self._mode)
         return _StyleGanAutoencoder(enc, dec, opts)
+
+    def _to_codes_cuda(self, batch: torch.Tensor, tape):
+        raise NotImplementedError("input gradient of to_codes through the Style-Transformer encoder: its attention, layer-norm and resize "
+                                  "backward are not built (to_codes without a gradient works)")
 
     def _encode(self, x_nhwc):
         ae = self.autoencoder

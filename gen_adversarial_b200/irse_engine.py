@@ -12,6 +12,11 @@ emits BN(x) as a second bf16 output, so no extra pass exists); `MaxPool2d(1, str
 sub-sample; the 1x1 stride-2 shortcut convs and the 3x3 stride-2 convs run on the tensor-core kernel with TMA element
 strides; `EqualLinear` scales folded; the learned query `z` of the Style-Transformer goes through the mapping MLP once
 for its 16 rows (the reference expands it to B x 16 rows first, style_transformer.py:57-61 / models.py:311-315).
+
+Input gradient (E4E; attacks): `IrSe50Backbone.backward` and `E4EEncoderEngine.encode_backward` run the dgrad-only reverse sweep over what a
+taped forward (`EncoderTape`) kept: per unit the PReLU output h of conv1, the conv2 output r and its SE channel sums, plus the stem output
+and every map2style activation.  The PReLU / LeakyReLU derivatives are recovered from the SIGN of those outputs (exact while every slope is
+> 0, checked when the dgrad layers are built); the BN in front of each unit's conv1 is folded into conv1's dgrad weights.
 """
 from __future__ import annotations
 
@@ -21,8 +26,9 @@ from typing import Dict, List, Optional
 import torch
 
 from . import ops
-from ._lib import PRE_NONE, PRE_AFFINE, ACT_NONE, ACT_RELU, ACT_PRELU
+from ._lib import PRE_NONE, PRE_AFFINE, ACT_NONE, ACT_RELU, ACT_PRELU, MUL_PRELU_FROM_Y
 from .fold import Folder
+from .resnet_engine import conv_dgrad
 
 IRSE50_BLOCKS = [(64, 64, 3), (64, 128, 4), (128, 256, 14), (256, 512, 3)]      # helpers.py:30-37 (in, depth, units)
 
@@ -37,7 +43,17 @@ def irse50_units():
 
 
 class _Unit:
-    __slots__ = ("cin", "depth", "stride", "pre", "c1", "c2", "sc", "se")
+    __slots__ = ("cin", "depth", "stride", "pre", "pre_scale64", "c1", "c2", "sc", "se", "c1_d", "c2_d", "sc_d")
+
+
+class EncoderTape:
+    """what a taped `E4EEncoderEngine.encode` keeps for `encode_backward` (tensors the forward produces anyway; nothing is recomputed)"""
+
+    def __init__(self):
+        self.stem = None          # stem output (PReLU output: unit 0's input and the stem's mask)
+        self.units = []           # per unit (h, r, sums): conv1's PReLU output, conv2's output, r's SE channel sums
+        self.heads = []           # per map2style head: the output of each conv (LeakyReLU outputs)
+        self.tap_shapes = None    # shapes of c1 / c2 / c3
 
 
 def conv1x1_any(engine, x, L, want_f32=False, add=None, out=None):
@@ -73,6 +89,7 @@ class IrSe50Backbone:
             p = f"body.{i}"
             a0, b0 = f.bn(f"{p}.res_layer.0")
             u.pre = (f.dev32(a0), f.dev32(b0))
+            u.pre_scale64 = a0
             u.c1 = f.conv(f.f64(f"{p}.res_layer.1.weight"), None, pad=1, pre_op=PRE_AFFINE, pre_affine=(a0, b0),
                           post_act=ACT_PRELU, name=f"{p}.conv1", tf32=self.tf32)
             u.c1.act_slope = f.dev32(f.f64(f"{p}.res_layer.2.weight"))
@@ -89,6 +106,7 @@ class IrSe50Backbone:
             w2 = f.f64(f"{p}.res_layer.5.fc2.weight").flatten(1)
             u.se = (f.dev32(w1), None, f.dev32(w2), None)
             self.units.append(u)
+        self._has_dgrad = False
 
     def _conv(self, x, L, want_f32=False, add=None, out=None):
         if self.bf16 and x.dtype == torch.float32 and L.w_tf32 is not None and ops.conv2d_tc_supported(x, L, tf32=True):
@@ -101,12 +119,15 @@ class IrSe50Backbone:
             return of if want_f32 else ob
         return ops.conv2d_simt(x, L, torch.float32 if (want_f32 or not self.bf16) else torch.bfloat16, add=add, out=out)
 
-    def forward(self, x_nhwc: torch.Tensor):
-        """x_nhwc (N,H,W,3) normalised input in the activation dtype -> (c1, c2, c3) in the activation dtype"""
+    def forward(self, x_nhwc: torch.Tensor, tape: Optional[EncoderTape] = None):
+        """x_nhwc (N,H,W,3) normalised input in the activation dtype -> (c1, c2, c3) in the activation dtype.
+        tape: an EncoderTape receiving what `backward` needs (build_dgrad() first); the values computed do not depend on it."""
         units = self.units
         x32 = ops.conv2d_simt(x_nhwc, self.stem, torch.float32)
+        if tape is not None:
+            tape.stem = x32
         if self.tf32:
-            return self._forward_tf32(x32)
+            return self._forward_tf32(x32, tape)
         xa = ops.affine_act(x32, units[0].pre[0], units[0].pre[1], ACT_NONE, torch.bfloat16) if self.bf16 else None
         xb = ops.cast(x32, torch.bfloat16) if (self.bf16 and units[0].sc is not None) else None
         taps = {}
@@ -124,6 +145,8 @@ class IrSe50Backbone:
             else:
                 skip = x32 if u.stride == 1 else ops.subsample2x(x32)
             sums = ops.channel_sum(r)
+            if tape is not None:
+                tape.units.append((h, r, sums))
             nxt = units[i + 1] if i + 1 < len(units) else None
             is_tap = i in (6, 20, 23)
             want_b = self.bf16 and (is_tap or (nxt is not None and nxt.sc is not None))
@@ -155,7 +178,7 @@ class IrSe50Backbone:
         finally:
             ops.f32_round_tf32(False)
 
-    def _forward_tf32(self, x32):
+    def _forward_tf32(self, x32, tape=None):
         units = self.units
         # BN of the first unit (the conv pads AFTER it), rounded to TF32
         xa = self._rounded(lambda: ops.affine_act(x32, units[0].pre[0], units[0].pre[1], ACT_NONE, torch.float32))
@@ -175,6 +198,8 @@ class IrSe50Backbone:
             else:
                 skip = x32 if u.stride == 1 else ops.subsample2x(x32)
             sums = ops.channel_sum(r)
+            if tape is not None:
+                tape.units.append((h, r, sums))
             nxt = units[i + 1] if i + 1 < len(units) else None
             is_tap = i in (6, 20, 23)
             x32, xb, xa, _ = self._rounded(lambda: ops.se_residual(
@@ -186,9 +211,54 @@ class IrSe50Backbone:
         self.c3_f32 = x32
         return taps[6], taps[20], taps[23]
 
+    # ------------------------------------------------------------------ input gradient
+    def build_dgrad(self, device):
+        """dgrad layers of the stem and the 24 units (built on the first taped forward: forward-only use pays nothing).  The PReLU masks are
+        recovered from the sign of the PReLU outputs, which is exact only for slopes > 0: any other slope refuses the backward."""
+        if self._has_dgrad:
+            return
+        from .nvae_engine import make_dgrad_layer
+        for L in [self.stem] + [u.c1 for u in self.units]:
+            if bool((L.act_slope <= 0).any()):
+                raise NotImplementedError(f"input gradient through the IR-SE50 backbone: PReLU of {L.name} has a slope <= 0, so its derivative "
+                                          f"cannot be recovered from the sign of its taped output")
+        f = Folder({}, device, want_tc=self.bf16)
+        for i, u in enumerate(self.units):
+            u.c1_d = make_dgrad_layer(f, u.c1, self.bf16, in_scale=u.pre_scale64)      # BN pre-affine (zero padding after it): scale folded
+            u.c1_d.act_slope = self.stem.act_slope if i == 0 else None                 # unit 0's input is the stem's PReLU output
+            u.c2_d = make_dgrad_layer(f, u.c2, self.bf16)
+            u.c2_d.act_slope = u.c1.act_slope                                          # mask of h = PReLU(conv1)
+            u.sc_d = make_dgrad_layer(f, u.sc, self.bf16) if u.sc is not None else None
+        self.stem_d = make_dgrad_layer(f, self.stem, self.bf16)
+        self._has_dgrad = True
+
+    def backward(self, tape: EncoderTape, g_c1: torch.Tensor, g_c2: torch.Tensor, g_c3: torch.Tensor) -> torch.Tensor:
+        """d loss / d (c1, c2, c3) fp32 NHWC -> d loss / d x_nhwc (N,H,W,3) fp32 (w.r.t. the normalised image); the residual-stream gradient
+        stays fp32, the gradients that only feed a dgrad conv are bf16 in bf16 mode.  The tape is left intact."""
+        dg = lambda g, D, **kw: conv_dgrad(g, D, self.bf16, mul_mode=MUL_PRELU_FROM_Y, **kw)
+        tap_grads = {6: g_c1, 20: g_c2, 23: g_c3}
+        g = None
+        for i in range(len(self.units) - 1, -1, -1):
+            u = self.units[i]
+            h, r, sums = tape.units[i]
+            t = tap_grads.get(i)
+            if t is not None:
+                g = t.contiguous() if g is None else ops.add(g, t.contiguous(), torch.float32)
+            g_r = ops.se_residual_bwd(g, r, sums, u.se, 1.0, self.adt)                 # the skip gradient is g itself
+            g_h = dg(g_r, u.c2_d, mul=h)                                                # times PReLU'(conv1) from the sign of h
+            if u.sc is not None:
+                g_skip = dg(g, u.sc_d, f32=True)                                        # 1x1 stride-2 shortcut
+            elif u.stride == 2:
+                g_skip = ops.subsample2x_bwd(g, (h.shape[1], h.shape[2]))               # MaxPool2d(1, 2)
+            else:
+                g_skip = g
+            # unit 0: times the stem's PReLU' (its output is unit 0's input), after the shortcut gradient has joined
+            g = dg(g_h, u.c1_d, add=g_skip, mul=tape.stem if i == 0 else None, f32=True)
+        return ops.conv2d_simt(g, self.stem_d, torch.float32)
+
 
 class _Head:
-    __slots__ = ("convs", "linear")
+    __slots__ = ("convs", "linear", "convs_d", "linear_d")
 
 
 class E4EEncoderEngine:
@@ -229,10 +299,29 @@ class E4EEncoderEngine:
         self.lat1 = f.conv(f.f64("latlayer1.weight"), f.f64("latlayer1.bias"), name="latlayer1", tf32=self.tf32_heads)
         self.lat2 = f.conv(f.f64("latlayer2.weight"), f.f64("latlayer2.bias"), name="latlayer2", tf32=self.tf32_heads)
         self.latent_avg = None if latent_avg is None else latent_avg.to(torch.float32).reshape(-1, 512)[: self.style_count].contiguous().to(self.device)
+        self._has_dgrad = False
 
     _conv = IrSe50Backbone._conv
 
-    def _head(self, feat, hd: _Head, out):
+    def build_dgrad(self):
+        """dgrad layers of the backbone, the FPN laterals and the heads (raises NotImplementedError for a PReLU slope <= 0, see
+        IrSe50Backbone.build_dgrad); called by the first taped `encode`"""
+        if self._has_dgrad:
+            return
+        from .nvae_engine import make_dgrad_layer
+        self.backbone.build_dgrad(self.device)
+        f = Folder({}, self.device, want_tc=self.bf16)
+        for hd in self.heads:
+            hd.convs_d = [make_dgrad_layer(f, L, self.bf16) for L in hd.convs]
+            for D in hd.convs_d[1:]:
+                D.act_slope = self.slope                          # its input is the previous conv's LeakyReLU output
+            hd.linear_d = make_dgrad_layer(f, hd.linear, self.bf16)
+            hd.linear_d.act_slope = self.slope
+        self.lat1_d = make_dgrad_layer(f, self.lat1, self.bf16)
+        self.lat2_d = make_dgrad_layer(f, self.lat2, self.bf16)
+        self._has_dgrad = True
+
+    def _head(self, feat, hd: _Head, out, acts=None):
         """map2style head.  bf16 mode: the final EqualLinear (and, optionally, the convs on maps <= fp32_tail_hw) run in fp32"""
         x = feat
         for L in hd.convs:
@@ -242,12 +331,19 @@ class E4EEncoderEngine:
                 x = ops.conv2d_simt(x, L, torch.float32)
             else:
                 x = self._conv(x, L)
+            if acts is not None:
+                acts.append(x)
         ops.conv2d_simt(x.reshape(x.shape[0], 1, 1, -1), hd.linear, torch.float32, out=out)
 
-    def encode(self, x_nhwc: torch.Tensor) -> torch.Tensor:
-        """x_nhwc (B,256,256,3) normalised -> codes (B, n_styles, 512) fp32 (latent_avg already added, psp.py:92-99)"""
+    def encode(self, x_nhwc: torch.Tensor, tape: Optional[EncoderTape] = None) -> torch.Tensor:
+        """x_nhwc (B,256,256,3) normalised -> codes (B, n_styles, 512) fp32 (latent_avg already added, psp.py:92-99).
+        tape: an EncoderTape to fill for encode_backward (the codes are the same with and without it)."""
         b = x_nhwc.shape[0]
-        c1, c2, c3 = self.backbone.forward(x_nhwc)
+        if tape is not None:
+            self.build_dgrad()
+        c1, c2, c3 = self.backbone.forward(x_nhwc, tape)
+        if tape is not None:
+            tape.tap_shapes = (c1.shape, c2.shape, c3.shape)
         rnd = IrSe50Backbone._rounded if self.tf32_heads else (lambda fn: fn())
         if self.tf32_heads and c3.dtype != torch.float32:
             c1, c2, c3 = (ops.cast(t, torch.float32) for t in (c1, c2, c3))          # bf16 values are exact in TF32
@@ -261,8 +357,41 @@ class E4EEncoderEngine:
             elif i == self.middle_ind:
                 feat = rnd(lambda: conv1x1_any(self, c1, self.lat2, add=ops.upsample_bilinear2x(p2), want_f32=self.tf32_heads))
             # head 0 (w0, added to all 18 codes) runs in fp32 from the fp32 residual stream in both modes: 1% of the encoder's FLOPs
-            self._head(self.backbone.c3_f32 if (i < self.fp32_heads and self.bf16) else feat, hd, heads[i])
+            acts = [] if tape is not None else None
+            self._head(self.backbone.c3_f32 if (i < self.fp32_heads and self.bf16) else feat, hd, heads[i], acts)
+            if tape is not None:
+                tape.heads.append(acts)
         return ops.codes_assemble(heads, True, True, self.latent_avg, b, self.style_count, 512)
+
+    def encode_backward(self, tape: EncoderTape, g_codes: torch.Tensor) -> torch.Tensor:
+        """g_codes (B, n_styles, 512) fp32 -> d loss / d x_nhwc (B,256,256,3) fp32 (w.r.t. the normalised image).  The heads' gradients are
+        summed per feature map (c3 / p2 / p1) in head order, each added in the epilogue of the head's last dgrad."""
+        dg = lambda g, D, **kw: conv_dgrad(g, D, self.bf16, mul_mode=MUL_PRELU_FROM_Y, **kw)
+        b = g_codes.shape[0]
+        g_heads = ops.codes_assemble_bwd(g_codes.to(torch.float32))                    # (n_styles, B, 512): w0 collects every code's gradient
+        g_feat = [None, None, None]                                                    # c3, p2, p1
+        for i, hd in enumerate(self.heads):
+            k = 0 if i < self.coarse_ind else (1 if i < self.middle_ind else 2)
+            acts = tape.heads[i]
+            g = dg(g_heads[i].reshape(b, 1, 1, 512), hd.linear_d, mul=acts[-1])        # EqualLinear transpose x LeakyReLU'
+            for j in range(len(hd.convs_d) - 1, 0, -1):
+                g = dg(g, hd.convs_d[j], mul=acts[j - 1])
+            g_feat[k] = dg(g, hd.convs_d[0], add=g_feat[k], f32=True)
+        g_c3, g_p2, g_p1 = g_feat
+        # _upsample_add: p2 = lat1(c2) + up(c3), p1 = lat2(c1) + up(p2)   (align_corners=True bilinear x2)
+        s1, s2, _ = tape.tap_shapes
+        if g_p1 is not None:
+            g_c1 = dg(g_p1, self.lat2_d, f32=True)
+            up = ops.upsample_bilinear2x_bwd(g_p1, torch.float32)
+            g_p2 = up if g_p2 is None else ops.add(g_p2, up, torch.float32)
+        else:
+            g_c1 = torch.zeros(s1, device=g_codes.device, dtype=torch.float32)
+        if g_p2 is not None:
+            g_c2 = dg(g_p2, self.lat1_d, f32=True)
+            g_c3 = ops.add(g_c3, ops.upsample_bilinear2x_bwd(g_p2, torch.float32), torch.float32)
+        else:
+            g_c2 = torch.zeros(s2, device=g_codes.device, dtype=torch.float32)
+        return self.backbone.backward(tape, g_c1, g_c2, g_c3)
 
 
 class _TLayer:

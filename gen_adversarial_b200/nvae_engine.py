@@ -46,11 +46,16 @@ def stride2_dgrad_phase_weights(w: torch.Tensor, pad: int) -> torch.Tensor:
     return wd.reshape(4 * cin, cout, k, k)
 
 
-def make_dgrad_layer(f: Folder, L: ops.ConvLayer, bf16: bool, pad_cin_to: Optional[int] = None) -> ops.ConvLayer:
+def make_dgrad_layer(f: Folder, L: ops.ConvLayer, bf16: bool, pad_cin_to: Optional[int] = None,
+                     in_scale: Optional[torch.Tensor] = None) -> ops.ConvLayer:
     """Input-gradient layer of the forward conv L (weights frozen: dgrad only): flipped taps, transposed channels; a stride-2 forward conv
     becomes an input-dilated (`up`) conv for the SIMT kernel and, in bf16 mode, ONE stride-1 tensor-core conv emitting the four output
-    phases (`.phase`, see stride2_dgrad_phase_weights).  pad_cin_to: zero-pad the dgrad's input channels (= forward cout) to this many."""
+    phases (`.phase`, see stride2_dgrad_phase_weights).  pad_cin_to: zero-pad the dgrad's input channels (= forward cout) to this many.
+    in_scale: fp64 [cin], the scale of a per-channel affine applied to L's input BEFORE its zero padding (L's PRE_AFFINE); its adjoint
+    scales the dgrad's output channels, folded into the weights here (exact: the padding follows the affine, so no border term exists)."""
     w = L.w_simt.detach().to("cpu", torch.float64).view(L.kh, L.kw, L.cin, L.cout).permute(3, 2, 0, 1)   # [cout,cin,kh,kw]
+    if in_scale is not None:
+        w = w * in_scale.to(torch.float64).view(1, -1, 1, 1)
     if pad_cin_to is not None and pad_cin_to > w.shape[0]:
         w = torch.cat([w, torch.zeros((pad_cin_to - w.shape[0],) + tuple(w.shape[1:]), dtype=w.dtype)], dim=0)
     wt = w.flip(2, 3).permute(1, 0, 2, 3).contiguous()           # [cin, cout(_pad), kh, kw]

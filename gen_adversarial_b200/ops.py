@@ -14,7 +14,7 @@ import torch
 
 from . import _lib
 from ._lib import GaTensor, GaConvDesc, GA_F32, GA_BF16, PRE_NONE, PRE_ELU, PRE_SILU, PRE_AFFINE_SILU, \
-    ACT_NONE, ACT_SILU, ACT_ELU, ACT_RELU, ACT_LRELU_SQRT2, MUL_VALUE, MUL_RELU_MASK, MUL_ELU_FROM_Y
+    ACT_NONE, ACT_SILU, ACT_ELU, ACT_RELU, ACT_LRELU_SQRT2, MUL_VALUE, MUL_RELU_MASK, MUL_ELU_FROM_Y, MUL_PRELU_FROM_Y
 
 
 def _dt(t: torch.Tensor) -> int:
@@ -727,6 +727,34 @@ def depth_to_space2(x: torch.Tensor) -> torch.Tensor:
     n, h, w, c4 = x.shape
     out = torch.empty((n, 2 * h, 2 * w, c4 // 4), device=x.device, dtype=torch.float32)
     _lib.check(_lib.lib().ga_depth_to_space2(gt(x), gt(out), stream()), "depth_to_space2")
+    return out
+
+
+@_timed("phase_interleave", hbm=True)
+def phase_interleave(x: torch.Tensor, add=None, mul=None, mul_mode: int = MUL_VALUE, slope=None, out_dtype=torch.float32) -> torch.Tensor:
+    """[n,h,w,4c] fp32 (phase-major channels) -> (depth_to_space2(x) + add) * f(mul) [n,2h,2w,c] in out_dtype, one pass; f is the
+    ga_mul_mode factor (MUL_PRELU_FROM_Y: `slope` [c] fp32, the slopes of the layer that produced `mul`)"""
+    n, h, w, c4 = x.shape
+    out = torch.empty((n, 2 * h, 2 * w, c4 // 4), device=x.device, dtype=out_dtype)
+    _lib.check(_lib.lib().ga_phase_interleave(gt(x), gt(add), gt(mul), int(mul_mode), ptr(slope), gt(out), stream()), "phase_interleave")
+    return out
+
+
+@_timed("subsample2x_bwd", hbm=True)
+def subsample2x_bwd(g: torch.Tensor, out_hw, out_dtype=torch.float32) -> torch.Tensor:
+    """adjoint of subsample2x: g [n,h,w,c] -> [n,H,W,c] with g at the even pixels, zeros elsewhere"""
+    out = torch.empty((g.shape[0], out_hw[0], out_hw[1], g.shape[3]), device=g.device, dtype=out_dtype)
+    _lib.check(_lib.lib().ga_subsample2x_bwd(gt(g), gt(out), stream()), "subsample2x_bwd")
+    return out
+
+
+@_timed("codes_assemble_bwd")
+def codes_assemble_bwd(g_codes: torch.Tensor) -> torch.Tensor:
+    """adjoint of codes_assemble(heads_lb=True, use_w0=True): g_codes (b, l, d) fp32 -> g_heads (l, b, d) fp32"""
+    b, l, d = g_codes.shape
+    g_codes = g_codes.contiguous()
+    out = torch.empty((l, b, d), device=g_codes.device, dtype=torch.float32)
+    _lib.check(_lib.lib().ga_codes_assemble_bwd(ptr(g_codes), b, l, d, ptr(out), stream()), "codes_assemble_bwd")
     return out
 
 

@@ -37,6 +37,33 @@ def densify_grouped(w: torch.Tensor, groups: int) -> torch.Tensor:
     return dense
 
 
+def conv_dgrad(g, D: ops.ConvLayer, bf16: bool, add=None, mul=None, f32: bool = False, mul_mode: int = MUL_RELU_MASK):
+    """input gradient through one conv (D from make_dgrad_layer): (dgrad(g) + add) * f(mul), f the mul_mode derivative of the activation whose
+    output `mul` is (MUL_PRELU_FROM_Y: D.act_slope holds that activation's slopes).  fp32 mode: SIMT fp32.  bf16 mode: tensor cores on a bf16
+    copy of g where the shape tiles, SIMT elsewhere; the output is bf16, or fp32 with f32 (gradients that join the residual stream)."""
+    if not bf16:
+        out_hw = (g.shape[1] * D.up, g.shape[2] * D.up) if D.up > 1 else None
+        return ops.conv2d_simt(g, D, torch.float32, add=add, out_hw=out_hw, mul=mul, mul_mode=mul_mode)
+    if g.dtype != torch.bfloat16:
+        g = ops.cast(g, torch.bfloat16)
+    if D.phase is not None and ops.conv2d_tc_supported(g, D.phase):
+        # stride-2 forward conv: the four output phases as one stride-1 tensor-core conv over g, interleaved, then add / mask
+        _, o4 = ops.conv2d_tc(g, D.phase, want_bf16=False, want_f32=True)
+        if mul_mode != MUL_RELU_MASK:                  # one fused pass (the ReLU-masked classifier path keeps its measured three passes)
+            return ops.phase_interleave(o4, add, mul, mul_mode, D.act_slope, torch.float32 if f32 else torch.bfloat16)
+        o = ops.depth_to_space2(o4)
+        if add is not None:
+            o = ops.add(o, add, torch.float32)
+        if mul is not None:
+            o = ops.affine_act_bwd(o, mul, None, None, ACT_RELU, torch.float32 if f32 else torch.bfloat16)
+        return o
+    if D.w_tc is not None and ops.conv2d_tc_supported(g, D):
+        ob, of = ops.conv2d_tc(g, D, want_bf16=not f32, want_f32=f32, add=add, mul=mul, mul_mode=mul_mode)
+        return of if f32 else ob
+    out_hw = (g.shape[1] * D.up, g.shape[2] * D.up) if D.up > 1 else None
+    return ops.conv2d_simt(g, D, torch.float32 if f32 else torch.bfloat16, add=add, out_hw=out_hw, mul=mul, mul_mode=mul_mode)
+
+
 class ResNetEngine:
     def __init__(self, state_dict: Dict[str, torch.Tensor], device, mode: str = "fp32", groups: int = 1,
                  _host_logic_test: bool = False):
@@ -121,26 +148,7 @@ class ResNetEngine:
 
     def _dg(self, g, D, add=None, mul=None, f32=False):
         """input gradient through one conv: (dgrad(g) + add) * [mul > 0]  (mul = the ReLU output that fed the forward conv)"""
-        mode = MUL_RELU_MASK
-        if not self.bf16:
-            out_hw = (g.shape[1] * D.up, g.shape[2] * D.up) if D.up > 1 else None
-            return ops.conv2d_simt(g, D, torch.float32, add=add, out_hw=out_hw, mul=mul, mul_mode=mode)
-        if g.dtype != torch.bfloat16:
-            g = ops.cast(g, torch.bfloat16)
-        if D.phase is not None:
-            # stride-2 forward conv: the four output phases as one stride-1 tensor-core conv over g, interleaved, then add / mask
-            _, o4 = ops.conv2d_tc(g, D.phase, want_bf16=False, want_f32=True)
-            o = ops.depth_to_space2(o4)
-            if add is not None:
-                o = ops.add(o, add, torch.float32)
-            if mul is not None:
-                o = ops.affine_act_bwd(o, mul, None, None, ACT_RELU, torch.float32 if f32 else torch.bfloat16)
-            return o
-        if D.w_tc is not None and ops.conv2d_tc_supported(g, D):
-            ob, of = ops.conv2d_tc(g, D, want_bf16=not f32, want_f32=f32, add=add, mul=mul, mul_mode=mode)
-            return of if f32 else ob
-        out_hw = (g.shape[1] * D.up, g.shape[2] * D.up) if D.up > 1 else None
-        return ops.conv2d_simt(g, D, torch.float32 if f32 else torch.bfloat16, add=add, out_hw=out_hw, mul=mul, mul_mode=mode)
+        return conv_dgrad(g, D, self.bf16, add=add, mul=mul, f32=f32)
 
     def backward(self, tape, g_logits: torch.Tensor) -> torch.Tensor:
         """g_logits (N, classes) fp32 -> d loss / d x_nhwc (N,H,W,3) fp32.  `tape` = the list filled by forward(tape=...)."""

@@ -34,9 +34,10 @@ enum ga_pre_op { GA_PRE_NONE = 0, GA_PRE_ELU = 1, GA_PRE_SILU = 2, GA_PRE_AFFINE
 enum ga_act { GA_ACT_NONE = 0, GA_ACT_SILU = 1, GA_ACT_ELU = 2, GA_ACT_RELU = 3,
               GA_ACT_LRELU_SQRT2 = 4 /* leaky_relu(x, 0.2) * sqrt(2): fused_bias_act_kernel.cu:28-47 */,
               GA_ACT_PRELU = 5 /* x > 0 ? x : act_slope[c] * x (nn.PReLU / nn.LeakyReLU of the IR-SE50 encoder) */ };
-/* epilogue multiplier modes (backward): multiply by the tensor itself, or by the ReLU / ELU derivative
- * reconstructed from the saved OUTPUT y of the forward activation (relu: y>0, elu: y>0 ? 1 : y+1) */
-enum ga_mul_mode { GA_MUL_VALUE = 0, GA_MUL_RELU_MASK = 1, GA_MUL_ELU_FROM_Y = 2 };
+/* epilogue multiplier modes (backward): multiply by the tensor itself, or by the ReLU / ELU / PReLU derivative
+ * reconstructed from the saved OUTPUT y of the forward activation (relu: y>0, elu: y>0 ? 1 : y+1, prelu: y>0 ? 1 : act_slope[c];
+ * for PReLU the desc's act_slope holds the slopes of the layer that produced y, which must all be > 0 for sign(y) = sign(x)) */
+enum ga_mul_mode { GA_MUL_VALUE = 0, GA_MUL_RELU_MASK = 1, GA_MUL_ELU_FROM_Y = 2, GA_MUL_PRELU_FROM_Y = 3 };
 
 /* dense NHWC tensor view */
 typedef struct ga_tensor {
@@ -308,7 +309,7 @@ int ga_affine_act_bwd(const ga_tensor* g, const ga_tensor* x, const float* scale
                       const ga_tensor* add /*nullable*/, const ga_tensor* out, void* stream);
 int ga_add(const ga_tensor* a, const ga_tensor* b, const ga_tensor* out, void* stream);
 /* backward of ga_se_residual_fwd w.r.t. r (the skip gradient is g_out itself): g_r = s*gate*g_out + d(gate MLP)/HW.
- * sums = the forward's partial channel sums of r; dots_ws = workspace of the same size. */
+ * sums = the forward's partial channel sums of r; dots_ws = workspace of the same size; b1 / b2 nullable (no bias). */
 int ga_se_residual_bwd(const ga_tensor* g_out, const ga_tensor* r, const float* sums, float* dots_ws, const float* w1,
                        const float* b1, const float* w2, const float* b2, int hidden, float res_scale,
                        const ga_tensor* g_r, void* stream);
@@ -318,6 +319,15 @@ int ga_upsample_bilinear2x_bwd(const ga_tensor* g_out, const ga_tensor* g_in, vo
  * convolution's input gradient, computed as one stride-1 tensor-core conv over grad_out (replaces the zero-stuffed SIMT transposed conv;
  * reference: autograd of the stride-2 convs of architecture.py:64-82,96-136) */
 int ga_depth_to_space2(const ga_tensor* in, const ga_tensor* out, void* stream);
+/* depth_to_space2 fused with the rest of a stride-2 dgrad epilogue, one pass: out = (d2s(in) + add) * f(mul) (ga_mul_mode; slope =
+ * act_slope [c] for GA_MUL_PRELU_FROM_Y), in fp32 [n,h,w,4c] -> out fp32 or bf16 [n,2h,2w,c]; add / mul nullable, out's shape */
+int ga_phase_interleave(const ga_tensor* in, const ga_tensor* add, const ga_tensor* mul, int mul_mode, const float* slope,
+                        const ga_tensor* out, void* stream);
+/* adjoint of ga_subsample2x (MaxPool2d(1, 2)): out[n][2y][2x][c] = g[n][y][x][c], zeros at the odd pixels */
+int ga_subsample2x_bwd(const ga_tensor* g, const ga_tensor* out, void* stream);
+/* adjoint of ga_codes_assemble(heads_lb = 1, use_w0 = 1) without the constant latent_avg: g_heads [l][b][d] from g_codes [b][l][d],
+ * g_heads[l] = g_codes[:, l] for l > 0, g_heads[0] = sum over l of g_codes[:, l] (fixed order, no atomics) */
+int ga_codes_assemble_bwd(const float* g_codes, int b, int l, int d, float* g_heads, void* stream);
 /* gradient to the first maximal element of each window (torch semantics); relu=1 also applies the mask x_in > 0 */
 int ga_maxpool2x2_bwd(const ga_tensor* x_in, const ga_tensor* g_out, int relu, const ga_tensor* g_in, void* stream);
 /* ResNet / ResNeXt classifier backward (SURVEY 8f rank 3): 3x3 stride-2 pad-1 max-pool backward (first maximum wins; relu: also the ReLU
